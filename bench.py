@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the neighbour-aggregation hot path (BASELINE.json).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME] ...
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME] [--dump-outputs DIR] ...
 
 N = 1 (default): BASELINE.json configs[1] -- the fused GCN layer H = (A X) W, feat 128 -> 128, on the
 synthetic reddit-shaped power-law graph (232,965 vertices / 114,615,891 edges), one B200.
@@ -21,6 +21,11 @@ A "step" = one pass of the layer over the whole graph.  Reported metric: algorit
 `value`: inputs resident in HBM; `e2e`: the same step with pinned HOST X/W/H and the copies inside the timed
 region (gnnagg_gcn_layer_host at N = 1).  `--impl reference`: the reference has no CPU implementation of this
 path (SURVEY 8(c)); the arm times the scalar CPU port (oracle/) on all host threads on a bounded sample.
+
+`--dump-outputs DIR` writes the layer output H of the last timed step as DIR/H.npy (float32).  The inputs are a pure
+function of the arguments (seeded graph and features), so two builds run with the same arguments can be compared
+output for output; an output larger than DUMP_BYTES is written as a fixed, seeded row sample.  At N > 1 every rank
+writes its own row block as DIR/H_rank<r>.npy.  The option belongs to the GPU path: `--impl reference` refuses it.
 """
 import argparse
 import json
@@ -47,6 +52,7 @@ WORKLOADS = {
 RMAT_SCALES = {"rmat26": (1 << 26, 1 << 30), "rmat22": (1 << 22, 1 << 26)}
 C5_WORKLOAD = "rmat26_gcn_agg_64"
 NVLINK_PEAK_GBS = 770.0  # measured peer-copy bandwidth per direction per GPU (B200_PROFILING.md); nominal 900
+DUMP_BYTES = 48 << 20    # --dump-outputs: at most this many bytes of output in all (split over the ranks)
 
 
 def layer_bytes(n, m, fin, fout):
@@ -377,9 +383,23 @@ def max_over_ranks(x, dev, dist):
     return float(t.item())
 
 
-def measure(wl, timed, steps, warmup, e2e=True):
+def output_sample(Y, budget_bytes, seed=0):
+    """what a caller of the timed path receives, copied to the host: the whole output when it fits in budget_bytes,
+    else a fixed row sample (rows drawn by numpy default_rng(seed) without replacement, in ascending order) -- the same
+    rows on every run with the same arguments.  Returns (array, description)."""
+    import numpy as np
+
+    n, F = Y.shape
+    k = min(n, max(1, budget_bytes // (Y.element_size() * F)))
+    if k == n:
+        return Y.cpu().numpy(), "all %d rows" % n
+    rows = np.sort(np.random.default_rng(seed).choice(n, k, replace=False))
+    return Y[rows].cpu().numpy(), "%d of %d rows, drawn by numpy default_rng(%d).choice(n, k, replace=False), sorted" % (k, n, seed)
+
+
+def measure(wl, timed, steps, warmup, e2e=True, dump_bytes=0):
     """times one workload: step, kernels-only step, exchange span, (optionally) end-to-end.  Collective: every rank
-    calls it."""
+    calls it.  dump_bytes > 0: out["output"] = output_sample() of what the last timed step computed."""
     import numpy as np
 
     out = {}
@@ -397,6 +417,8 @@ def measure(wl, timed, steps, warmup, e2e=True):
         ms = timed(wl.step, steps, warmup)
     out["launches_per_step"] = (wl.launch_count() - l0) / float(steps + warmup)
     out["ms"] = ms
+    if dump_bytes > 0:  # taken before the passes below run the layer again
+        out["output"] = output_sample(wl.H, dump_bytes)
     out["prof"] = {k: float(np.mean([p[k] for p in prof])) for k in prof[0]} if prof else {}
     if wl.N > 1:
         out["compute_ms"] = timed(lambda: wl.step(exchange=False), max(3, steps // 2), 2)
@@ -564,7 +586,14 @@ def main():
                                                         "with the default workload)")
     ap.add_argument("--c5-sweep", default="", help="comma-separated remote-stage counts for the c5 block")
     ap.add_argument("--ref-kernels", type=int, default=1, help="N=1: time the reference's own kernels (oracle/_ref) after the headline")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the headline output of the last timed step as DIR/H.npy (float32; a fixed row sample when "
+                         "it exceeds %d MiB; one file per rank, H_rank<r>.npy, at N > 1)" % (DUMP_BYTES >> 20))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's output: not with --impl reference")
     args.warmup = max(args.warmup, 3)
 
     import numpy as np
@@ -674,8 +703,18 @@ def main():
                 del w2
                 torch.cuda.empty_cache()
 
-    r = measure(wl, timed, args.steps, args.warmup, e2e=True)
+    r = measure(wl, timed, args.steps, args.warmup, e2e=True, dump_bytes=DUMP_BYTES // N if args.dump_outputs else 0)
     clocks = sampler.result()
+    dumped = None
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        name = "H" if N == 1 else "H_rank%d" % rank
+        H, how = r["output"]
+        np.save(os.path.join(args.dump_outputs, name + ".npy"), H)
+        # printed by rank 0: every rank's file is listed, the details are those of rank 0's (the others have the same
+        # dtype and width, and their rows are sampled the same way from their own row blocks)
+        dumped = {"dir": args.dump_outputs, "files": ["H.npy"] if N == 1 else ["H_rank%d.npy" % q for q in range(N)],
+                  name: {"dtype": str(H.dtype), "shape": list(H.shape), "rows": how}}
     timed, barrier = make_timer(dev, dist, None, flush)  # the clock sampler covers the headline region only
     ms, ms_e2e = r["ms"], r["ms_e2e"]
     parity = parity_check(wl) if N > 1 else None
@@ -783,6 +822,8 @@ def main():
                                      ", the library's own CUDA events" if N == 1 else ", timed like the step with the exchange switched off, max over ranks")},
                 "roofline": roofline, "cpu_baseline": cpu_baseline,
                 "setup_s": round(wl.setup_s, 2)}
+        if dumped is not None:
+            line["outputs_dumped"] = dumped
         if N > 1:
             line["e2e"]["copies_only_ms"] = round(r["ms_copies"], 4)
             line["e2e"]["note"] = "copies_only_ms = the H2D + D2H of the same buffers alone, all ranks at once: what the host side of this box allows at this N"
