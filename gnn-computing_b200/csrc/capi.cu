@@ -90,6 +90,13 @@ constexpr double kLocalityMinL2Multiples = 8.0;
 constexpr double kLocalitySliceL2Multiples = 2.5;
 constexpr double kLocalityMinDegree = 20.0;
 constexpr int kLocalityMaxAuto = 4;
+// automatic merged view of duplicate edges (gnnagg_set_merge_duplicates(a, 0)), DESIGN.md §4.11: merging must remove at
+// least kMergeMinFraction of the edges (reddit / proteins shapes: 34 %, 16-28 % faster layer; arxiv / products shapes:
+// 5 %, no gain beyond the spread), on graphs of at least kMergeMinEdges edges -- the small-graph bound of
+// kSmallGraphEdges, below which the aggregation is bound by the length of one warp's walk rather than by the L1 data
+// path that merging relieves, and where the decision's host synchronisation would fall on every small aggregator
+constexpr int64_t kMergeMinEdges = 4000000;
+constexpr double kMergeMinFraction = 0.10;
 
 struct gnnagg_aggregator {
     // borrowed graph
@@ -166,6 +173,14 @@ struct gnnagg_aggregator {
     cudaStream_t in_stream = nullptr;
     cudaEvent_t in_done[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     cudaEvent_t in_free = nullptr;
+    // merged view (gnnagg_set_merge_duplicates): runs of adjacent equal sources in a row as one entry each.  `mg` runs
+    // over mg_ptr / mg_idx / mg_val (owned here) with its own item table, carry and long-row records; built on first use
+    int merge_mode = 0;       // 0 = automatic, 1 = off, 2 = on
+    int merge_auto = -1;      // automatic decision: -1 not taken yet, 0 off, 1 on
+    gnnagg_aggregator *mg = nullptr;
+    int *mg_ptr = nullptr, *mg_idx = nullptr, *mg_start = nullptr;  // mg_start[k]: CSR edge id of run k's first edge
+    float *mg_val = nullptr;
+    const float *mg_val_of = nullptr;  // which d_val mg_val currently sums (NULL: none / stale after gnnagg_set_val)
     // optional per-kernel timing (gnnagg_profile_enable)
     bool prof = false;
     cudaEvent_t ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};  // begin, agg0, agg1, agg_end, end
@@ -243,6 +258,18 @@ __global__ void scatter_val_kernel(const float *__restrict__ in, const int *__re
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < count) out[__ldg(perm + i)] = __ldg(in + i);
+}
+
+// val'[k] = sum of the values of run k in CSR order, in fp64, rounded once; one thread per run (deterministic)
+__global__ void merge_val_kernel(const float *__restrict__ val, const int *__restrict__ start, float *__restrict__ out,
+                                 int runs)
+{
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= runs) return;
+    const int end = __ldg(start + k + 1);
+    double s = 0.0;
+    for (int e = __ldg(start + k); e < end; ++e) s += (double)__ldg(val + e);
+    out[k] = (float)s;
 }
 
 static int check_feat(int F)
@@ -591,6 +618,7 @@ static int mlp_run_core(gnnagg_aggregator *a, const float *P, float *Y, int F, i
 }
 
 static void free_slices(gnnagg_aggregator *a);
+static int merged_view(gnnagg_aggregator *a, cudaStream_t st, gnnagg_aggregator **out);
 
 // builds the source slices on first use and (re)mirrors the edge values into slice order
 static int ensure_slices(gnnagg_aggregator *a, int want, cudaStream_t st, bool compact = false)
@@ -706,8 +734,14 @@ static int gcn_run_impl(gnnagg_aggregator *a, const float *X, float *Y, int F, i
     if (S > 1) {
         if (!aligned16(X) || !aligned16(Y)) return set_error(GNNAGG_ERR_ARG, "X and Y must be 16-byte aligned");
         if (int rc = gcn_run_sliced(a, X, Y, F, S, st, accumulate)) return rc;
-    } else if (int rc = gcn_run_core(a, X, Y, F, scheduled, st, accumulate)) {
-        return rc;
+    } else {
+        gnnagg_aggregator *t = a;
+        if (a && !scheduled)
+            if (int rc = merged_view(a, st, &t)) return rc;
+        const int64_t before = t ? t->launches : 0;
+        const int rc = gcn_run_core(t, X, Y, F, scheduled, st, accumulate);
+        if (t != a) a->launches += t->launches - before;
+        if (rc) return rc;
     }
     PROF_RECORD(a, 3, st);
     if (last) PROF_RECORD(a, 4, st);
@@ -800,6 +834,89 @@ static void free_transpose(gnnagg_aggregator *a)
     a->num_src = 0;
 }
 
+static void free_merged(gnnagg_aggregator *a)
+{
+    if (a->mg) {
+        cudaFree(a->mg->d_item_row);
+        cudaFree(a->mg->carry);
+        free_long_rows(a->mg);
+        delete a->mg;  // its timing events are the parent's
+        a->mg = nullptr;
+    }
+    cudaFree(a->mg_ptr), cudaFree(a->mg_idx), cudaFree(a->mg_start), cudaFree(a->mg_val);
+    a->mg_ptr = a->mg_idx = a->mg_start = nullptr;
+    a->mg_val = nullptr;
+    a->mg_val_of = nullptr;
+}
+
+// whether the un-scheduled, un-sliced GCN aggregation runs on the merged view (after ensure_merged)
+static bool merged_in_use(const gnnagg_aggregator *a)
+{
+    return a->mg && (a->merge_mode == 2 || (a->merge_mode == 0 && a->merge_auto == 1));
+}
+
+// builds the merged view when the setting asks for it; automatic: takes the decision once (kMergeMin*) from a count of
+// m', so that a graph the rule leaves alone pays one counting pass and no m-sized allocation
+static int ensure_merged(gnnagg_aggregator *a, cudaStream_t st)
+{
+    if (a->merge_mode == 1 || a->n == 0 || a->m == 0) return GNNAGG_OK;
+    if (a->merge_mode == 0 && a->merge_auto < 0) {
+        int mm = a->m;
+        if (a->m >= kMergeMinEdges) {
+            if (int rc = merge_count_device(a->d_ptr, a->d_idx, a->n, a->m, &mm, st)) return rc;
+            a->launches += 2;
+        }
+        a->merge_auto = (double)(a->m - mm) >= kMergeMinFraction * (double)a->m && a->m >= kMergeMinEdges;
+    }
+    if (a->merge_mode == 0 && a->merge_auto == 0) return GNNAGG_OK;
+    if (!a->mg) {
+        int mm = 0;
+        if (int rc = merge_build_device(a->d_ptr, a->d_idx, a->n, a->m, &a->mg_ptr, &a->mg_idx, &a->mg_start, &mm, st))
+            return rc;
+        a->launches += 5;  // run heads, row heads, scan (counted once), compaction, row pointers
+        if (cudaMalloc((void **)&a->mg_val, (size_t)(mm ? mm : 1) * sizeof(float)) != cudaSuccess) {
+            free_merged(a);
+            return set_error(GNNAGG_ERR_CUDA, "merged view: out of device memory");
+        }
+        gnnagg_aggregator *g = new gnnagg_aggregator();
+        g->d_ptr = a->mg_ptr;
+        g->d_idx = a->mg_idx;
+        g->d_val = a->mg_val;
+        g->n = a->n;
+        g->m = mm;
+        g->merge_mode = 1;
+        a->mg = g;
+        if (int rc = build_item_rows(g, g->d_ptr, g->n, g->m, &g->d_item_row, &g->num_items, st)) {
+            free_merged(a);
+            return rc;
+        }
+        a->launches += g->launches;
+        g->launches = 0;
+    }
+    return GNNAGG_OK;
+}
+
+// the aggregator the un-scheduled, un-sliced GCN aggregation of `a` runs on: the merged view when it is in use (its
+// values re-summed on `st` when the edge values changed), else `a` itself
+static int merged_view(gnnagg_aggregator *a, cudaStream_t st, gnnagg_aggregator **out)
+{
+    *out = a;
+    if (a->merge_mode == 1 || !a->d_val) return GNNAGG_OK;
+    if (int rc = ensure_merged(a, st)) return rc;
+    if (!merged_in_use(a)) return GNNAGG_OK;
+    gnnagg_aggregator *g = a->mg;
+    if (a->mg_val_of != a->d_val) {
+        merge_val_kernel<<<(unsigned)cdiv(g->m, 256), 256, 0, st>>>(a->d_val, a->mg_start, a->mg_val, g->m);
+        LAUNCH_CHECK(a);
+        a->mg_val_of = a->d_val;
+    }
+    g->warp_edges = a->warp_edges;
+    g->prof = a->prof;  // the aggregation kernel's events are the parent's (gnnagg_profile_read)
+    for (int i = 0; i < 5; ++i) g->ev[i] = a->ev[i];
+    *out = g;
+    return GNNAGG_OK;
+}
+
 // t_val[j] = src[t_perm[j]]: edge data into transposed order
 static int to_transposed(gnnagg_aggregator *a, const float *src, float *dst, cudaStream_t st)
 {
@@ -874,6 +991,7 @@ int gnnagg_destroy(gnnagg_aggregator *a)
         delete a->loc;
         a->loc = nullptr;
     }
+    free_merged(a);
     free_long_rows(a);
     for (int i = 0; i < 8; ++i)
         if (a->in_done[i]) cudaEventDestroy(a->in_done[i]);
@@ -917,6 +1035,7 @@ int gnnagg_set_val_on(gnnagg_aggregator *a, const float *d_val, void *stream)
     a->d_val = d_val;
     a->t_val_of = nullptr;  // same pointer, possibly new contents (aggr_gcn.h:540-544): re-mirror on the next backward
     a->sl_val_of = nullptr;
+    a->mg_val_of = nullptr;
     if (a->loc) a->loc->sl_val_of = nullptr;
     if (a->sched_kind == GNNAGG_SCHED_NOP) return GNNAGG_OK;
     if (a->s_perm) {  // locality kinds keep a permuted copy (aggr_gcn.h:522-537)
@@ -1018,6 +1137,29 @@ int gnnagg_set_locality_slices(gnnagg_aggregator *a, int slices)
     return GNNAGG_OK;
 }
 
+int gnnagg_set_merge_duplicates(gnnagg_aggregator *a, int mode)
+{
+    if (!a || mode < 0 || mode > 2) return set_error(GNNAGG_ERR_ARG, "gnnagg_set_merge_duplicates: 0 (automatic), 1 (off), 2 (on)");
+    a->merge_mode = mode;  // a view already built stays until gnnagg_destroy: switching back costs no rebuild
+    return GNNAGG_OK;
+}
+
+int gnnagg_merged_edges(gnnagg_aggregator *a)
+{
+    if (!a) return set_error(-1, "gnnagg_merged_edges: NULL aggregator");
+    if (ensure_merged(a, nullptr) != GNNAGG_OK) return -1;
+    return merged_in_use(a) ? a->mg->m : a->m;
+}
+
+int gnnagg_merged_dev(const gnnagg_aggregator *a, const int **ptr, const int **idx, const float **val)
+{
+    if (!a || !merged_in_use(a)) return set_error(GNNAGG_ERR_STATE, "gnnagg_merged_dev: the merged view is not in use");
+    if (ptr) *ptr = a->mg_ptr;
+    if (idx) *idx = a->mg_idx;
+    if (val) *val = a->mg_val;
+    return GNNAGG_OK;
+}
+
 int gnnagg_profile_enable(gnnagg_aggregator *a, int on)
 {
     if (!a) return set_error(GNNAGG_ERR_ARG, "gnnagg_profile_enable: NULL aggregator");
@@ -1056,6 +1198,14 @@ int gnnagg_prepare(gnnagg_aggregator *a, int feat, void *stream)
     if (!a) return set_error(GNNAGG_ERR_ARG, "gnnagg_prepare: NULL aggregator");
     if (int rc = check_feat(feat)) return rc;
     if (a->m == 0 || a->n == 0) return GNNAGG_OK;
+    gnnagg_aggregator *t = a;
+    if (int rc = merged_view(a, (cudaStream_t)stream, &t)) return rc;
+    if (t != a) {
+        const int64_t before = t->launches;
+        const int rc = gnnagg_prepare(t, feat, stream);
+        a->launches += t->launches - before;
+        return rc;
+    }
     const int EB = item_edges_for(a, feat, a->m);
     if (int rc = ensure(a->carry, a->carry_cap, (size_t)cdiv(a->m, EB) * feat)) return rc;
     if (warp_edges_for(a, a->m) == 128)
@@ -1084,9 +1234,14 @@ int gnnagg_gcn_run_rows(gnnagg_aggregator *a, const float *X, float *Y, int feat
     if (!a) return set_error(GNNAGG_ERR_ARG, "gnnagg_gcn_run_rows: NULL aggregator");
     if (row_lo < 0 || row_hi > a->n || row_lo > row_hi) return set_error(GNNAGG_ERR_ARG, "gnnagg_gcn_run_rows: bad row range");
     if (row_lo == row_hi) return GNNAGG_OK;
+    gnnagg_aggregator *t = a;
+    if (int rc = merged_view(a, (cudaStream_t)stream, &t)) return rc;
     const int *hp = nullptr;
-    if (int rc = host_ptr(a, &hp)) return rc;
-    return gcn_run_core(a, X, Y, feat, 0, (cudaStream_t)stream, accumulate != 0, row_lo, row_hi, hp[row_lo], hp[row_hi]);
+    if (int rc = host_ptr(t, &hp)) return rc;
+    const int64_t before = t->launches;
+    const int rc = gcn_run_core(t, X, Y, feat, 0, (cudaStream_t)stream, accumulate != 0, row_lo, row_hi, hp[row_lo], hp[row_hi]);
+    if (t != a) a->launches += t->launches - before;
+    return rc;
 }
 
 int gnnagg_gcn_run(gnnagg_aggregator *a, const float *X, float *Y, int feat, int scheduled, void *stream)
@@ -1570,6 +1725,7 @@ static int gcn_host_pipeline(gnnagg_aggregator *a, const float *h_X, const float
         tail[1] = a->slice[tail_first + 1];
     } else {
         CUDA_TRY(cudaMemcpyAsync(a->st_in, h_X, cin * sizeof(float), cudaMemcpyHostToDevice, st));
+        if (int rc = merged_view(a, st, &tail[0])) return rc;  // the rows gcn_run aggregates, chunk by chunk
     }
     const int *hp[2] = {nullptr, nullptr};
     for (int t = 0; t < tail_count; ++t)
@@ -1578,7 +1734,7 @@ static int gcn_host_pipeline(gnnagg_aggregator *a, const float *h_X, const float
     if (S > 1) {  // equal ROW counts: the chunks are sized for the copy back
         for (int c = 0; c <= kHostChunks; ++c) bounds[c] = (int)((int64_t)a->n * c / kHostChunks);
     } else {
-        row_chunks(hp[0], a->n, a->m, kHostChunks, bounds);
+        row_chunks(hp[0], a->n, tail[0]->m, kHostChunks, bounds);
     }
     for (int c = 0; c < kHostChunks; ++c) {
         const int r0 = bounds[c], r1 = bounds[c + 1];

@@ -986,6 +986,8 @@ int gnnagg_dist_set_graph(gnnagg_dist *d, const int *d_ptr, const int *d_idx, co
     for (int s = 0; s < d->num_stages; ++s) {
         rc = gnnagg_create(d->sl_ptr + (size_t)s * ((size_t)n + 1), d->sl_idx + d->sl_off[s], nullptr, nullptr, n, d->sl_cnt[s],
                            &d->stage[s]);
+        // stages run on their own CSR: the merged view of duplicate edges is not used across ranks (yet)
+        if (rc == GNNAGG_OK) rc = gnnagg_set_merge_duplicates(d->stage[s], 1);
         if (rc == GNNAGG_OK) rc = gnnagg_set_val(d->stage[s], d->sl_val + d->sl_off[s]);
         if (rc != GNNAGG_OK) {
             free_graph(d);

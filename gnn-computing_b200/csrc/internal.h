@@ -38,6 +38,13 @@ int source_slices_build_device(const int *d_ptr, const int *d_idx, const int *d_
 // non-empty rows of a sub-CSR and their row pointers (sched_device.cu); outputs are cudaMalloc'ed
 int compact_rows_device(const int *d_ptr, int n, int **c_ptr, int **c_row, int *n_out, cudaStream_t st);
 
+// runs of adjacent equal sources inside a row merged into one entry each (sched_device.cu); outputs are cudaMalloc'ed
+int merge_build_device(const int *d_ptr, const int *d_idx, int n, int m, int **mg_ptr, int **mg_idx, int **mg_start,
+                       int *merged_edges, cudaStream_t st);
+
+// m' of that merge, counted without building it (sched_device.cu)
+int merge_count_device(const int *d_ptr, const int *d_idx, int n, int m, int *merged_edges, cudaStream_t st);
+
 // item_row table of a CSR (row containing edge k*128), cudaMalloc'ed into *out (capi.cu)
 int build_item_rows_device(const int *d_ptr, int rows, int edges, int **out, int *items, cudaStream_t st);
 

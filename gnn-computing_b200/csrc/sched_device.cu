@@ -448,4 +448,124 @@ fail:
     return GNNAGG_ERR_CUDA;
 }
 
+
+// ---------------------------------------------------------------------------------------------------------
+// Merged view of a CSR (capi.cu: merged_view): every run of ADJACENT equal sources inside a row becomes one entry,
+// so the aggregation gathers each (row, source) pair once.  No sort, no reordering: a CSR sorted within its rows
+// merges every duplicate, an unsorted one the adjacent ones only.  The structure depends on ptr / idx alone; the
+// values are summed per run by merge_val_kernel whenever the edge values change.  Outputs (cudaMalloc'ed, owned by
+// the caller):
+//   *mg_ptr   [n+1]  merged row pointers, mg_ptr[r] = merged position of ptr[r]
+//   *mg_idx   [m']   the source of every run
+//   *mg_start [m'+1] CSR edge id of the first edge of every run; mg_start[m'] = m
+// ---------------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) run_head_kernel(const int *__restrict__ idx, int m, int *__restrict__ head)
+{
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e < m) head[e] = (e == 0 || __ldg(idx + e) != __ldg(idx + e - 1)) ? 1 : 0;
+    if (e == m) head[m] = 0;  // the exclusive scan then ends in the run count
+}
+
+// the first edge of every non-empty row starts a run (runs never cross a row boundary); after run_head_kernel
+__global__ void __launch_bounds__(256) row_head_kernel(const int *__restrict__ ptr, int n, int *__restrict__ head)
+{
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r < n && ptr[r] < ptr[r + 1]) head[ptr[r]] = 1;
+}
+
+__global__ void __launch_bounds__(256) run_compact_kernel(const int *__restrict__ idx, const int *__restrict__ head,
+                                                          const int *__restrict__ pos, int m, int *__restrict__ mg_idx,
+                                                          int *__restrict__ mg_start)
+{
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e < m && head[e]) {
+        mg_idx[pos[e]] = __ldg(idx + e);
+        mg_start[pos[e]] = e;
+    }
+    if (e == m) mg_start[pos[m]] = m;
+}
+
+__global__ void __launch_bounds__(256) merged_ptr_kernel(const int *__restrict__ ptr, const int *__restrict__ pos, int n,
+                                                         int *__restrict__ mg_ptr)
+{
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r <= n) mg_ptr[r] = pos[ptr[r]];
+}
+
+// m' without building anything: adjacent source changes, plus the first edge, plus the row starts whose source equals
+// the previous edge's (a run never crosses a row boundary).  Integer counts: the atomics are exact.
+__global__ void __launch_bounds__(256) count_changes_kernel(const int *__restrict__ idx, int m, int *__restrict__ count)
+{
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    const int c = (e < m && (e == 0 || __ldg(idx + e) != __ldg(idx + e - 1))) ? 1 : 0;
+    const int s = __syncthreads_count(c);
+    if (threadIdx.x == 0 && s) atomicAdd(count, s);
+}
+
+__global__ void __launch_bounds__(256) count_row_splits_kernel(const int *__restrict__ ptr, const int *__restrict__ idx, int n,
+                                                               int *__restrict__ count)
+{
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    int c = 0;
+    if (r < n) {
+        const int e = ptr[r];
+        c = (e > 0 && e < ptr[r + 1] && __ldg(idx + e) == __ldg(idx + e - 1)) ? 1 : 0;
+    }
+    const int s = __syncthreads_count(c);
+    if (threadIdx.x == 0 && s) atomicAdd(count, s);
+}
+
+int merge_count_device(const int *d_ptr, const int *d_idx, int n, int m, int *merged_edges, cudaStream_t st)
+{
+    *merged_edges = 0;
+    int *count = nullptr;
+    SD_TRY(cudaMalloc((void **)&count, sizeof(int)));
+    SD_TRY(cudaMemsetAsync(count, 0, sizeof(int), st));
+    if (m > 0) count_changes_kernel<<<blocks(m), 256, 0, st>>>(d_idx, m, count);
+    if (n > 0 && m > 0) count_row_splits_kernel<<<blocks(n), 256, 0, st>>>(d_ptr, d_idx, n, count);
+    SD_TRY(cudaGetLastError());
+    SD_TRY(cudaMemcpyAsync(merged_edges, count, sizeof(int), cudaMemcpyDeviceToHost, st));
+    SD_TRY(cudaStreamSynchronize(st));
+    cudaFree(count);
+    return GNNAGG_OK;
+fail:
+    cudaFree(count);
+    return GNNAGG_ERR_CUDA;
+}
+
+int merge_build_device(const int *d_ptr, const int *d_idx, int n, int m, int **mg_ptr, int **mg_idx, int **mg_start,
+                       int *merged_edges, cudaStream_t st)
+{
+    *mg_ptr = *mg_idx = *mg_start = nullptr;
+    *merged_edges = 0;
+    int *head = nullptr, *pos = nullptr;
+    void *tmp = nullptr;
+    size_t need = 0;
+    int mm = 0;
+    SD_TRY(cudaMalloc((void **)&head, ((size_t)m + 1) * sizeof(int)));
+    SD_TRY(cudaMalloc((void **)&pos, ((size_t)m + 1) * sizeof(int)));
+    run_head_kernel<<<blocks((int64_t)m + 1), 256, 0, st>>>(d_idx, m, head);
+    if (n > 0) row_head_kernel<<<blocks(n), 256, 0, st>>>(d_ptr, n, head);
+    SD_TRY(cub::DeviceScan::ExclusiveSum(nullptr, need, head, pos, m + 1, st));
+    SD_TRY(cudaMalloc(&tmp, need ? need : 1));
+    SD_TRY(cub::DeviceScan::ExclusiveSum(tmp, need, head, pos, m + 1, st));
+    SD_TRY(cudaMemcpyAsync(&mm, pos + m, sizeof(int), cudaMemcpyDeviceToHost, st));
+    SD_TRY(cudaStreamSynchronize(st));
+    SD_TRY(cudaMalloc((void **)mg_ptr, ((size_t)n + 1) * sizeof(int)));
+    SD_TRY(cudaMalloc((void **)mg_idx, (size_t)(mm > 0 ? mm : 1) * sizeof(int)));
+    SD_TRY(cudaMalloc((void **)mg_start, ((size_t)mm + 1) * sizeof(int)));
+    run_compact_kernel<<<blocks((int64_t)m + 1), 256, 0, st>>>(d_idx, head, pos, m, *mg_idx, *mg_start);
+    merged_ptr_kernel<<<blocks((int64_t)n + 1), 256, 0, st>>>(d_ptr, pos, n, *mg_ptr);
+    SD_TRY(cudaGetLastError());
+    SD_TRY(cudaStreamSynchronize(st));
+    *merged_edges = mm;
+    cudaFree(head), cudaFree(pos), cudaFree(tmp);
+    return GNNAGG_OK;
+fail:
+    cudaFree(head), cudaFree(pos), cudaFree(tmp);
+    cudaFree(*mg_ptr), cudaFree(*mg_idx), cudaFree(*mg_start);
+    *mg_ptr = *mg_idx = *mg_start = nullptr;
+    return GNNAGG_ERR_CUDA;
+}
+
 }  // namespace gnnagg

@@ -102,6 +102,9 @@ _SIGS = {
     "gnnagg_set_warp_edges": (C.c_int, [C.c_void_p, C.c_int]),
     "gnnagg_set_host_pipeline": (C.c_int, [C.c_void_p, C.c_int]),
     "gnnagg_set_locality_slices": (C.c_int, [C.c_void_p, C.c_int]),
+    "gnnagg_set_merge_duplicates": (C.c_int, [C.c_void_p, C.c_int]),
+    "gnnagg_merged_edges": (C.c_int, [C.c_void_p]),
+    "gnnagg_merged_dev": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_void_p)]),
     "gnnagg_profile_enable": (C.c_int, [C.c_void_p, C.c_int]),
     "gnnagg_profile_read": (C.c_int, [C.c_void_p, C.POINTER(C.c_float)]),
     "gnnagg_memcpy_d2h": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64]),
@@ -341,6 +344,38 @@ class Aggregator:
 
     def set_locality_slices(self, slices):
         check(lib().gnnagg_set_locality_slices(self.h, int(slices)))
+
+    def set_merge_duplicates(self, mode):
+        """0 automatic, 1 off, 2 on (gnnagg_set_merge_duplicates)"""
+        check(lib().gnnagg_set_merge_duplicates(self.h, int(mode)))
+
+    @property
+    def merged_edges(self):
+        """edges the GCN aggregation walks: m' of the merged view, or m when it is off"""
+        import torch
+
+        torch.cuda.current_stream().synchronize()  # the view is built on the legacy stream from ptr/idx
+        e = lib().gnnagg_merged_edges(self.h)
+        if e < 0:
+            raise GnnaggError("gnnagg_merged_edges: %s" % lib().gnnagg_last_error().decode(errors="replace"))
+        return e
+
+    def merged_arrays(self):
+        """the merged view as the last run left it, copied back as numpy (ptr, idx, val)"""
+        import torch
+
+        L = lib()
+        p, i, v = C.c_void_p(), C.c_void_p(), C.c_void_p()
+        check(L.gnnagg_merged_dev(self.h, C.byref(p), C.byref(i), C.byref(v)))
+        torch.cuda.synchronize()
+        mp = np.empty(self.n + 1, np.int32)
+        check(L.gnnagg_memcpy_d2h(mp.ctypes.data, p, mp.nbytes))
+        e = int(mp[-1])
+        mi, mv = np.empty(e, np.int32), np.empty(e, np.float32)
+        if e:
+            check(L.gnnagg_memcpy_d2h(mi.ctypes.data, i, mi.nbytes))
+            check(L.gnnagg_memcpy_d2h(mv.ctypes.data, v, mv.nbytes))
+        return mp, mi, mv
 
     def set_host_pipeline(self, slices):
         check(lib().gnnagg_set_host_pipeline(self.h, int(slices)))

@@ -120,6 +120,8 @@ class HaloPipeline:
         self.chunks = chunks
         parts = split_by_source_chunk(ptr, idx, val, n_per, world, rank, chunks)
         self.aggs = [Aggregator(p, i, v) for p, i, v in parts]
+        for agg in self.aggs:  # multi-GPU blocks keep their CSR as given (as the gnnagg_dist_* stages do)
+            agg.set_merge_duplicates(1)
         self.edges = [int(i.numel()) for _, i, _ in parts]
         self.Xc = [torch.empty((world * (self.cb[c + 1] - self.cb[c]), feat), device=ptr.device) for c in range(chunks)]
 
@@ -184,6 +186,7 @@ class PrunedHalo:
         self.send_buf = torch.empty((self.send_rows.numel(), feat), device=dev)
         self.recv_buf = torch.empty((self.num_recv, feat), device=dev)
         self.agg = Aggregator(ptr, self.idx_compact, val)
+        self.agg.set_merge_duplicates(1)  # multi-GPU blocks keep their CSR as given (as the gnnagg_dist_* stages do)
         self.referenced_fraction = self.num_recv / float(n_per * world)
 
     def exchange(self, Xs):
@@ -268,6 +271,7 @@ class PipelinedPrunedHalo:
             e0, e1 = int(hp[r0]), int(hp[r1])
             sub_ptr = (ptr[r0:r1 + 1] - e0).contiguous()
             self.aggs.append(Aggregator(sub_ptr, plan["idx_compact"][e0:e1].contiguous(), val[e0:e1].contiguous()))
+            self.aggs[-1].set_merge_duplicates(1)  # as above: multi-GPU blocks keep their CSR as given
             self.rows.append((r0, r1))
         self.send_rows = torch.cat(plan["send_rows"]) if chunks else torch.empty(0, dtype=torch.int64, device=dev)
         self.send_off = np.concatenate([[0], np.cumsum([t.numel() for t in plan["send_rows"]])]).astype(np.int64)

@@ -394,6 +394,25 @@ int gnnagg_set_host_pipeline(gnnagg_aggregator *a, int slices);
  * Results are deterministic for a given setting; slices change the fp32 summation order (slice by slice). */
 int gnnagg_set_locality_slices(gnnagg_aggregator *a, int slices);
 
+/* Merged view of duplicate edges for the un-scheduled, un-sliced GCN aggregation (gnnagg_gcn_run, gnnagg_gcn_run_acc,
+ * gnnagg_gcn_layer, gnnagg_gcn_run_rows and the row-chunk host pipeline): every run of ADJACENT edges of a row with the
+ * same source becomes one entry whose value is the run's sum (summed in fp64 in CSR order, rounded once to fp32), so
+ * each (row, source) pair is gathered once.  The same matrix A; built once on the GPU from ptr / idx (no sort, no
+ * reordering: rows sorted by source merge every duplicate), its values re-summed on the run's stream after
+ * gnnagg_set_val.  Scheduled runs, locality and source slices, GAT, SDDMM, MLP and the backward passes keep the CSR.
+ *   0  automatic (default): on when the graph has >= 4M edges and merging removes >= 10 % of them
+ *   1  off (the CSR as given);  2  on.
+ * Results are deterministic for a given setting; merging changes the fp32 summation order. */
+int gnnagg_set_merge_duplicates(gnnagg_aggregator *a, int mode);
+
+/* edges the GCN aggregation walks under the current setting: m' of the merged view, or num_e when it is off (builds
+ * the view, or takes the automatic decision, on the legacy stream if that has not happened yet); -1 on error */
+int gnnagg_merged_edges(gnnagg_aggregator *a);
+
+/* device arrays of the merged view (row pointers [num_v+1], sources [m'], values [m']) as the last run left them;
+ * GNNAGG_ERR_STATE when the view is not in use */
+int gnnagg_merged_dev(const gnnagg_aggregator *a, const int **ptr, const int **idx, const float **val);
+
 /* tuning knob (the reference's analogue is the BLOCK_SIZE argument of run(), aggr_gcn.h:381-386):
  * edges staged per warp by the aggregation kernels: 0 = automatic (128 below 4M edges, else 512),
  * or force 128 / 512.  Results do not depend on it beyond fp32 summation order. */
