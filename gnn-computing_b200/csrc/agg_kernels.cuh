@@ -21,6 +21,7 @@
 //   * 64-bit addressing of X/Y (the reference overflows int at idx*F, aggr_gcn.h:23).
 #pragma once
 #include <climits>
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -33,7 +34,7 @@ struct AggParams {
     const float *__restrict__ val;       // GCN edge values; unused for GAT
     const int *__restrict__ target;      // scheduled mode: output row of every group
     const int *__restrict__ item_row;    // row containing edge k*kFineItem
-    const float *__restrict__ X;         // [*, F]
+    const void *__restrict__ X;          // [*, F] fp32, or bf16 bit patterns for the XBF16 instances of the GCN mode
     const float *__restrict__ att;       // GAT attention table [n,2]
     const float *__restrict__ P;         // MLP: projected features P = X*W, [n, F] (also the gather source); SDDMM: X2
     float *__restrict__ Y;               // [n, F]
@@ -85,11 +86,27 @@ __device__ __forceinline__ int item_start_row(const AggParams &p, int e0)
     return row_of_edge(p.ptr, p.item_row, p.num_fine_items, p.num_rows, e0);
 }
 
+// four consecutive columns of the gathered row at x: a float4, or (XBF16) four bf16 in 8 bytes widened exactly to fp32
+// (a bf16 is the high half of an fp32)
+template <bool XBF16>
+__device__ __forceinline__ float4 ldg_x4(const char *x)
+{
+    if (!XBF16) return __ldg(reinterpret_cast<const float4 *>(x));
+    const uint2 h = __ldg(reinterpret_cast<const uint2 *>(x));
+    return make_float4(__uint_as_float(h.x << 16), __uint_as_float(h.x & 0xffff0000u), __uint_as_float(h.y << 16),
+                       __uint_as_float(h.y & 0xffff0000u));
+}
+
 // WE = edges staged per warp: 512 normally, 128 for small graphs (4x more warps, shorter walks)
 // (5 resident CTAs per SM for the small-graph variant -- 48 registers -- measured on the arxiv shape: no change.)
-template <int LPR, int NV, int MODE, bool SCHED, int WE>
+// XBF16 (GCN only): X holds bf16.  The lane mapping, items and carries are those of the fp32 run of the same width;
+// each lane gathers 8 bytes where it gathered 16 and runs the same FMAs on the widened values, so the result equals the
+// fp32 run on the widened X bit for bit.
+template <int LPR, int NV, int MODE, bool SCHED, int WE, bool XBF16 = false>
 __global__ void __launch_bounds__(kCtaThreads, (WE < 512) ? 4 : 3) agg_kernel(const AggParams p)
 {
+    static_assert(!XBF16 || MODE == kModeGCN, "bf16 X is a GCN-only operand");
+    using XT = typename std::conditional<XBF16, uint16_t, float>::type;
     constexpr int kWarpEdges = WE;            // shadows the namespace-level default
     constexpr int VPW = 32 / LPR;             // virtual warps per warp
     constexpr int EB = kWarpEdges / VPW;      // edges per item
@@ -259,10 +276,11 @@ __global__ void __launch_bounds__(kCtaThreads, (WE < 512) ? 4 : 3) agg_kernel(co
 
         // gather base of this lane: column `col` of row 0 (inactive lanes of a partial chunk read
         // column 0 instead of being predicated off; their results are never stored)
-        const char *xb = reinterpret_cast<const char *>(opaque64(reinterpret_cast<uint64_t>(p.X + (act0 ? col : 0))));
-        const uint32_t row_bytes = opaque32((uint32_t)F * 4u);
+        const char *xb = reinterpret_cast<const char *>(
+            opaque64(reinterpret_cast<uint64_t>(static_cast<const XT *>(p.X) + (act0 ? col : 0))));
+        const uint32_t row_bytes = opaque32((uint32_t)F * (uint32_t)sizeof(XT));
         const uint32_t s_base = opaque32(smem_u32(my_idx));  // shared address of this warp's staged idx (val: + 4*kWarpEdges)
-        const int second = act1 ? LPR * 16 : 0;  // byte offset of the second float4 (NV == 2)
+        const int second = act1 ? LPR * 4 * (int)sizeof(XT) : 0;  // byte offset of the second 4 columns (NV == 2)
 
         // per-edge outputs: lane emit_id * (LPR / U) of the virtual warp ends up with the total of edge emit_id of a batch
         const int emit_id = (int)opaque32((uint32_t)(vl / (LPR / U)));
@@ -406,8 +424,8 @@ __global__ void __launch_bounds__(kCtaThreads, (WE < 512) ? 4 : 3) agg_kernel(co
 #pragma unroll
             for (int u = 0; u < U; ++u) {
                 const char *x = xb + (size_t)(uint32_t)src[u] * row_bytes;
-                v0[u] = __ldg(reinterpret_cast<const float4 *>(x));
-                if (NV > 1) v1[u] = __ldg(reinterpret_cast<const float4 *>(x + second));
+                v0[u] = ldg_x4<XBF16>(x);
+                if (NV > 1) v1[u] = ldg_x4<XBF16>(x + second);
             }
             float wout = 0.f;
 #pragma unroll
@@ -465,8 +483,8 @@ __global__ void __launch_bounds__(kCtaThreads, (WE < 512) ? 4 : 3) agg_kernel(co
 #pragma unroll
             for (int u = 0; u < U; ++u) {
                 const char *x = xb + (size_t)(uint32_t)src[u] * row_bytes;  // one IMAD.WIDE.U32
-                v0[u] = __ldg(reinterpret_cast<const float4 *>(x));
-                if (NV > 1) v1[u] = __ldg(reinterpret_cast<const float4 *>(x + second));
+                v0[u] = ldg_x4<XBF16>(x);
+                if (NV > 1) v1[u] = ldg_x4<XBF16>(x + second);
             }
             float wout = 0.f;
             const bool whole = row_end - e >= U;  // no row ends inside the batch

@@ -361,19 +361,26 @@ static inline int item_edges_for(const View &v, int F, int64_t num_edges)
 
 using AggKernel = void (*)(const AggParams);
 
-// the aggregation kernel for a mode, edges per warp and feature width
-template <int MODE, bool SCHED>
+// the aggregation kernel for a mode, edges per warp, feature width and element type of X
+template <int MODE, bool SCHED, bool XBF16 = false>
 static AggKernel agg_kernel_for(int WE, int F)
 {
     if (WE == 128)
-        return F <= 32 ? agg_kernel<8, 1, MODE, SCHED, 128>
-             : F <= 64 ? agg_kernel<16, 1, MODE, SCHED, 128>
-             : F <= 128 ? agg_kernel<32, 1, MODE, SCHED, 128>
-                        : agg_kernel<32, 2, MODE, SCHED, 128>;
-    return F <= 32 ? agg_kernel<8, 1, MODE, SCHED, kWarpEdges>
-         : F <= 64 ? agg_kernel<16, 1, MODE, SCHED, kWarpEdges>
-         : F <= 128 ? agg_kernel<32, 1, MODE, SCHED, kWarpEdges>
-                    : agg_kernel<32, 2, MODE, SCHED, kWarpEdges>;
+        return F <= 32 ? agg_kernel<8, 1, MODE, SCHED, 128, XBF16>
+             : F <= 64 ? agg_kernel<16, 1, MODE, SCHED, 128, XBF16>
+             : F <= 128 ? agg_kernel<32, 1, MODE, SCHED, 128, XBF16>
+                        : agg_kernel<32, 2, MODE, SCHED, 128, XBF16>;
+    return F <= 32 ? agg_kernel<8, 1, MODE, SCHED, kWarpEdges, XBF16>
+         : F <= 64 ? agg_kernel<16, 1, MODE, SCHED, kWarpEdges, XBF16>
+         : F <= 128 ? agg_kernel<32, 1, MODE, SCHED, kWarpEdges, XBF16>
+                    : agg_kernel<32, 2, MODE, SCHED, kWarpEdges, XBF16>;
+}
+template <int MODE, bool SCHED>
+static AggKernel agg_kernel_for(int WE, int F, bool xbf16)
+{
+    if constexpr (MODE == kModeGCN)
+        if (xbf16) return agg_kernel_for<MODE, SCHED, true>(WE, F);
+    return agg_kernel_for<MODE, SCHED>(WE, F);
 }
 
 // CUDA loads a kernel lazily at its first launch, and that load can wait for the device to go idle.  A process that
@@ -416,8 +423,9 @@ static const LongRows *long_rows_of(View &v, const AggParams &p, int EB, cudaStr
     return &v.long_rows.back();
 }
 
+// xbf16: p.X holds bf16 (GCN only)
 template <int MODE, bool SCHED>
-static int launch_agg(View &v, AggParams p, cudaStream_t st)
+static int launch_agg(View &v, AggParams p, cudaStream_t st, bool xbf16 = false)
 {
     if (p.row_hi == 0 && p.edge_hi == 0) {  // callers that do not set a row range get the whole graph
         p.row_lo = 0, p.row_hi = p.num_rows, p.edge_lo = 0, p.edge_hi = p.num_edges;
@@ -428,7 +436,7 @@ static int launch_agg(View &v, AggParams p, cudaStream_t st)
     const int WE = warp_edges_for(v, p.num_edges);
     const int64_t first = (int64_t)(p.edge_lo / WE) * WE;  // warps keep their global 512-edge alignment (TMA staging)
     const unsigned grid = (unsigned)cdiv(p.edge_hi - first, (int64_t)WE * kCtaWarps);
-    const AggKernel kernel = agg_kernel_for<MODE, SCHED>(WE, p.F);
+    const AggKernel kernel = agg_kernel_for<MODE, SCHED>(WE, p.F, xbf16);
     if (MODE == kModeGATBWD || MODE == kModeGATBWD2)
         launch_dep(kernel, grid, kCtaThreads, st, p);
     else
@@ -457,6 +465,27 @@ static int launch_agg(View &v, AggParams p, cudaStream_t st)
 }
 
 static int aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
+// the gathered operand of a GCN aggregation: fp32 X (16-byte aligned), or bf16 bit patterns (8-byte aligned) that the
+// kernel widens exactly to fp32
+struct GatherX {
+    const void *p;
+    bool bf16;
+    GatherX(const float *x) : p(x), bf16(false) {}
+    GatherX(const uint16_t *x) : p(x), bf16(true) {}
+    int elem_bytes() const { return bf16 ? 2 : 4; }
+};
+
+static int check_xy(const GatherX &X, const float *Y)
+{
+    if (X.bf16) {
+        if ((reinterpret_cast<uintptr_t>(X.p) & 7) || !aligned16(Y))
+            return set_error(GNNAGG_ERR_ARG, "X (bf16) must be 8-byte aligned and Y 16-byte aligned");
+    } else if (!aligned16(X.p) || !aligned16(Y)) {
+        return set_error(GNNAGG_ERR_ARG, "X and Y must be 16-byte aligned");
+    }
+    return GNNAGG_OK;
+}
 
 // the traversal fields of AggParams: a view's CSR, or the root's schedule
 static void set_view(AggParams &p, const View &v)
@@ -491,16 +520,16 @@ static int sched_prologue(gnnagg_aggregator *a, float *Y, int F, cudaStream_t st
 
 // rows [row_lo, row_hi) of the un-scheduled aggregation over v (row_hi < 0: all rows); Y is indexed by GLOBAL row.
 // Scheduled runs use v.root's schedule.
-static int gcn_run_core(View &v, const float *X, float *Y, int F, int scheduled, cudaStream_t st, int accumulate = 0,
+static int gcn_run_core(View &v, GatherX X, float *Y, int F, int scheduled, cudaStream_t st, int accumulate = 0,
                         int row_lo = 0, int row_hi = -1, int edge_lo = 0, int edge_hi = 0)
 {
     if (v.n == 0) return GNNAGG_OK;  // an empty row block (possible after edge-balanced partitioning)
-    if (!X || !Y) return set_error(GNNAGG_ERR_ARG, "gnnagg_gcn_run: NULL argument");
+    if (!X.p || !Y) return set_error(GNNAGG_ERR_ARG, "gnnagg_gcn_run: NULL argument");
     if (int rc = check_feat(F)) return rc;
-    if (!aligned16(X) || !aligned16(Y)) return set_error(GNNAGG_ERR_ARG, "X and Y must be 16-byte aligned");
+    if (int rc = check_xy(X, Y)) return rc;
     if (!v.d_val && v.m > 0) return set_error(GNNAGG_ERR_STATE, "gnnagg_gcn_run: edge values not set (gnnagg_set_val)");
     AggParams p{};
-    p.X = X;
+    p.X = X.p;
     p.Y = Y;
     p.F = F;
     if (scheduled) {
@@ -508,7 +537,7 @@ static int gcn_run_core(View &v, const float *X, float *Y, int F, int scheduled,
         if (p.num_edges == 0) return GNNAGG_OK;
         p.val = v.root->sched.val;
         p.bulk_ok = aligned16(p.idx) && aligned16(p.val);
-        return launch_agg<kModeGCN, true>(v, p, st);
+        return launch_agg<kModeGCN, true>(v, p, st, X.bf16);
     }
     if (v.m == 0) {
         if (!accumulate) CUDA_TRY(cudaMemsetAsync(Y, 0, (size_t)v.n * F * sizeof(float), st));
@@ -530,7 +559,7 @@ static int gcn_run_core(View &v, const float *X, float *Y, int F, int scheduled,
             return GNNAGG_OK;
         }
     }
-    return launch_agg<kModeGCN, false>(v, p, st);
+    return launch_agg<kModeGCN, false>(v, p, st, X.bf16);
 }
 
 // host mirror of the row pointers (needed to cut row chunks)
@@ -690,7 +719,8 @@ static int ensure_slices(gnnagg_aggregator *a, std::unique_ptr<Slices> &set, int
 
 
 // how many source slices the device-resident un-scheduled aggregation uses for this feature width (1 = none)
-static int locality_slices_for(const gnnagg_aggregator *a, int F)
+// x_elem_bytes: bytes per element of X as stored (4 fp32, 2 bf16); the constants were tuned on fp32 runs only
+static int locality_slices_for(const gnnagg_aggregator *a, int F, int x_elem_bytes)
 {
     if (a->loc_slices >= 1) return a->loc_slices < kMaxSlices ? a->loc_slices : kMaxSlices;
     // automatic: worth it when X is many times the L2 (the gathers of a slice then stay resident where those of the
@@ -698,7 +728,7 @@ static int locality_slices_for(const gnnagg_aggregator *a, int F)
     int dev = 0, l2 = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&l2, cudaDevAttrL2CacheSize, dev) != cudaSuccess || l2 <= 0)
         return 1;
-    const double x_bytes = 4.0 * (double)a->n * F;
+    const double x_bytes = (double)x_elem_bytes * (double)a->n * F;
     if (x_bytes < kLocalityMinL2Multiples * (double)l2 || a->m < kSmallGraphEdges) return 1;
     if ((double)a->m < kLocalityMinDegree * (double)a->n) return 1;
     int S = (int)(x_bytes / (kLocalitySliceL2Multiples * (double)l2) + 0.999);
@@ -706,7 +736,7 @@ static int locality_slices_for(const gnnagg_aggregator *a, int F)
 }
 
 // Y (+)= A X slice by slice over the source ranges; same result as the un-sliced run up to fp32 summation order
-static int gcn_run_sliced(gnnagg_aggregator *a, const float *X, float *Y, int F, int S, cudaStream_t st, int accumulate)
+static int gcn_run_sliced(gnnagg_aggregator *a, GatherX X, float *Y, int F, int S, cudaStream_t st, int accumulate)
 {
     if (int rc = ensure_slices(a, a->loc, S, st, true)) return rc;
     PROF_RECORD(a, 1, st);
@@ -730,16 +760,17 @@ static int prof_agg_empty(gnnagg_aggregator *a, cudaStream_t st)
 static int merged_view(gnnagg_aggregator *a, cudaStream_t st, View **out);
 
 // timing brackets: ev[0] call entry, ev[3] end of the aggregation part, ev[4] end of the call
-static int gcn_run_impl(gnnagg_aggregator *a, const float *X, float *Y, int F, int scheduled, cudaStream_t st,
+static int gcn_run_impl(gnnagg_aggregator *a, GatherX X, float *Y, int F, int scheduled, cudaStream_t st,
                         bool last = true, int accumulate = 0)
 {
     if (!a) return set_error(GNNAGG_ERR_ARG, "gnnagg_gcn_run: NULL argument");
     PROF_RECORD(a, 0, st);
     if (int rc = prof_agg_empty(a, st)) return rc;
     int S = 1;
-    if (!scheduled && a->n > 0 && a->m > 0 && X && Y && check_feat(F) == GNNAGG_OK && a->d_val) S = locality_slices_for(a, F);
+    if (!scheduled && a->n > 0 && a->m > 0 && X.p && Y && check_feat(F) == GNNAGG_OK && a->d_val)
+        S = locality_slices_for(a, F, X.elem_bytes());
     if (S > 1) {
-        if (!aligned16(X) || !aligned16(Y)) return set_error(GNNAGG_ERR_ARG, "X and Y must be 16-byte aligned");
+        if (int rc = check_xy(X, Y)) return rc;
         if (int rc = gcn_run_sliced(a, X, Y, F, S, st, accumulate)) return rc;
     } else {
         View *t = a;
@@ -852,6 +883,40 @@ static int merged_view(gnnagg_aggregator *a, cudaStream_t st, View **out)
     g.v.warp_edges = a->warp_edges;  // the setting follows the root's; automatic decides on m'
     *out = &g.v;
     return GNNAGG_OK;
+}
+
+static int gcn_layer_impl(gnnagg_aggregator *a, GatherX X, const float *W, float *H, float *AX, int feat_in, int feat_out,
+                          int scheduled, void *stream)
+{
+    if (!a || !X.p || !W || !H) return set_error(GNNAGG_ERR_ARG, "gnnagg_gcn_layer: NULL argument");
+    float *ax = AX;
+    if (!ax) {
+        if (int rc = a->ax.ensure((size_t)a->n * feat_in)) return rc;
+        ax = a->ax.p;
+    }
+    if (int rc = gcn_run_impl(a, X, ax, feat_in, scheduled, (cudaStream_t)stream, false)) return rc;
+    if (a->n > 0) {
+        if (int rc = dense_nn_launch(ax, W, H, a->n, feat_out, feat_in, stream)) return rc;
+        a->launches += 2;  // split_w_kernel + dense_tf32x3_ws_kernel
+    }
+    PROF_RECORD(a, 4, (cudaStream_t)stream);
+    return GNNAGG_OK;
+}
+
+static int gcn_backward_impl(gnnagg_aggregator *a, GatherX dY, float *dX, int feat, cudaStream_t st)
+{
+    if (!a || !dY.p || !dX) return set_error(GNNAGG_ERR_ARG, "gnnagg_gcn_backward: NULL argument");
+    if (!a->tr) return set_error(GNNAGG_ERR_STATE, "gnnagg_gcn_backward: gnnagg_transpose_build has not run");
+    if (!a->d_val && a->m > 0) return set_error(GNNAGG_ERR_STATE, "gnnagg_gcn_backward: edge values not set (gnnagg_set_val)");
+    Transpose &t = *a->tr;
+    if (t.val_gen != a->val_gen) {  // t.val[j] = val[perm[j]]: the edge values in transposed order
+        if (a->m > 0) {
+            gather_val_kernel<<<(unsigned)cdiv(a->m, 256), 256, 0, st>>>(a->d_val, t.perm.p, t.val.p, a->m);
+            LAUNCH_CHECK(a);
+        }
+        t.val_gen = a->val_gen;
+    }
+    return gcn_run_core(t.v, dY, dX, feat, 0, st);
 }
 
 }  // namespace gnnagg
@@ -1085,6 +1150,7 @@ int gnnagg_prepare(gnnagg_aggregator *a, int feat, void *stream)
     const int EB = item_edges_for(v, feat, v.m);
     if (int rc = v.carry.ensure((size_t)cdiv(v.m, EB) * feat)) return rc;
     preload(agg_kernel_for<kModeGCN, false>(warp_edges_for(v, v.m), feat));
+    preload(agg_kernel_for<kModeGCN, false, true>(warp_edges_for(v, v.m), feat));  // gnnagg_gcn_run_bf16
     preload(agg_fixup_kernel<kModeGCN>);
     preload(agg_fixup_long_kernel<kModeGCN>);
     AggParams p{};
@@ -1112,6 +1178,11 @@ int gnnagg_gcn_run(gnnagg_aggregator *a, const float *X, float *Y, int feat, int
     return gcn_run_impl(a, X, Y, feat, scheduled, (cudaStream_t)stream);
 }
 
+int gnnagg_gcn_run_bf16(gnnagg_aggregator *a, const uint16_t *X, float *Y, int feat, int scheduled, void *stream)
+{
+    return gcn_run_impl(a, X, Y, feat, scheduled, (cudaStream_t)stream);
+}
+
 int gnnagg_gcn_run_acc(gnnagg_aggregator *a, const float *X, float *Y, int feat, int accumulate, void *stream)
 {
     return gcn_run_impl(a, X, Y, feat, 0, (cudaStream_t)stream, true, accumulate != 0);
@@ -1133,19 +1204,13 @@ int gnnagg_dense_nn(const float *A, const float *B, float *C, int64_t M, int N, 
 int gnnagg_gcn_layer(gnnagg_aggregator *a, const float *X, const float *W, float *H, float *AX, int feat_in,
                      int feat_out, int scheduled, void *stream)
 {
-    if (!a || !X || !W || !H) return set_error(GNNAGG_ERR_ARG, "gnnagg_gcn_layer: NULL argument");
-    float *ax = AX;
-    if (!ax) {
-        if (int rc = a->ax.ensure((size_t)a->n * feat_in)) return rc;
-        ax = a->ax.p;
-    }
-    if (int rc = gcn_run_impl(a, X, ax, feat_in, scheduled, (cudaStream_t)stream, false)) return rc;
-    if (a->n > 0) {
-        if (int rc = dense_nn_launch(ax, W, H, a->n, feat_out, feat_in, stream)) return rc;
-        a->launches += 2;  // split_w_kernel + dense_tf32x3_ws_kernel
-    }
-    PROF_RECORD(a, 4, (cudaStream_t)stream);
-    return GNNAGG_OK;
+    return gcn_layer_impl(a, X, W, H, AX, feat_in, feat_out, scheduled, stream);
+}
+
+int gnnagg_gcn_layer_bf16(gnnagg_aggregator *a, const uint16_t *X, const float *W, float *H, float *AX, int feat_in,
+                          int feat_out, int scheduled, void *stream)
+{
+    return gcn_layer_impl(a, X, W, H, AX, feat_in, feat_out, scheduled, stream);
 }
 
 int gnnagg_mlp_run(gnnagg_aggregator *a, const float *X, const float *W, float *Y, int feat, int scheduled,
@@ -1303,19 +1368,12 @@ int gnnagg_transpose_dev(const gnnagg_aggregator *a, int *num_src, const int **t
 
 int gnnagg_gcn_backward(gnnagg_aggregator *a, const float *dY, float *dX, int feat, void *stream)
 {
-    if (!a || !dY || !dX) return set_error(GNNAGG_ERR_ARG, "gnnagg_gcn_backward: NULL argument");
-    if (!a->tr) return set_error(GNNAGG_ERR_STATE, "gnnagg_gcn_backward: gnnagg_transpose_build has not run");
-    if (!a->d_val && a->m > 0) return set_error(GNNAGG_ERR_STATE, "gnnagg_gcn_backward: edge values not set (gnnagg_set_val)");
-    cudaStream_t st = (cudaStream_t)stream;
-    Transpose &t = *a->tr;
-    if (t.val_gen != a->val_gen) {  // t.val[j] = val[perm[j]]: the edge values in transposed order
-        if (a->m > 0) {
-            gather_val_kernel<<<(unsigned)cdiv(a->m, 256), 256, 0, st>>>(a->d_val, t.perm.p, t.val.p, a->m);
-            LAUNCH_CHECK(a);
-        }
-        t.val_gen = a->val_gen;
-    }
-    return gcn_run_core(t.v, dY, dX, feat, 0, st);
+    return gcn_backward_impl(a, dY, dX, feat, (cudaStream_t)stream);
+}
+
+int gnnagg_gcn_backward_bf16(gnnagg_aggregator *a, const uint16_t *dY, float *dX, int feat, void *stream)
+{
+    return gcn_backward_impl(a, dY, dX, feat, (cudaStream_t)stream);
 }
 
 int gnnagg_gat_backward(gnnagg_aggregator *a, const float *X, const float *att, const float *w, const float *den,

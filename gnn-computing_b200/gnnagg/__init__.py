@@ -69,11 +69,13 @@ _SIGS = {
     "gnnagg_sched_dev_val": (C.c_void_p, [C.c_void_p]),
     "gnnagg_prepare": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
     "gnnagg_gcn_run": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
+    "gnnagg_gcn_run_bf16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "gnnagg_gcn_run_rows": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "gnnagg_gcn_run_acc": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "gnnagg_gcn_run_edgewise": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "gnnagg_csr2edgelist": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "gnnagg_gcn_layer": (C.c_int, [C.c_void_p] * 5 + [C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "gnnagg_gcn_layer_bf16": (C.c_int, [C.c_void_p] * 5 + [C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "gnnagg_dense_nn": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p]),
     "gnnagg_gat_run": (C.c_int, [C.c_void_p] * 4 + [C.c_int, C.c_float, C.c_int, C.c_void_p]),
     "gnnagg_gat_edge_weights": (C.c_void_p, [C.c_void_p]),
@@ -86,6 +88,7 @@ _SIGS = {
     "gnnagg_transpose_build": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
     "gnnagg_transpose_dev": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)] + [C.POINTER(C.c_void_p)] * 3),
     "gnnagg_gcn_backward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
+    "gnnagg_gcn_backward_bf16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "gnnagg_gat_backward": (C.c_int, [C.c_void_p] * 9 + [C.c_int, C.c_float, C.c_void_p]),
     "gnnagg_sample_subgraph": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_uint64] + [C.POINTER(C.c_void_p)] * 3 +
                                [C.POINTER(C.c_int)] * 2 + [C.c_void_p]),
@@ -275,6 +278,26 @@ def _f32(t, name, cuda=True):
     return C.c_void_p(t.data_ptr())
 
 
+def _bf16(t, name):
+    """device bfloat16 operand (the gathered X / dY of the bf16 GCN entry points); numpy has no bf16, so there is
+    no host path"""
+    import torch
+
+    if t.dtype != torch.bfloat16:
+        raise GnnaggError("%s: expected bfloat16, got %s" % (name, t.dtype))
+    if not t.is_contiguous():
+        raise GnnaggError("%s: expected a contiguous row-major tensor (got strides %s)" % (name, tuple(t.stride())))
+    if not t.is_cuda:
+        raise GnnaggError("%s: expected a CUDA tensor" % name)
+    return C.c_void_p(t.data_ptr())
+
+
+def _is_bf16(t):
+    import torch
+
+    return not isinstance(t, np.ndarray) and t.dtype == torch.bfloat16
+
+
 def device_info():
     sm, ma, mi = C.c_int(), C.c_int(), C.c_int()
     name = C.create_string_buffer(256)
@@ -408,9 +431,12 @@ class Aggregator:
         sv = back(pv, e, np.float32) if pv else None
         return sp, si, stt, sv
 
-    # --- GCN
+    # --- GCN (gcn_run, gcn_layer and gcn_backward take a float32 or a bfloat16 X / dY; outputs are float32)
     def gcn_run(self, X, Y, scheduled=False):
-        check(lib().gnnagg_gcn_run(self.h, _f32(X, "X"), _f32(Y, "Y"), X.shape[1], int(scheduled), _stream()))
+        if _is_bf16(X):
+            check(lib().gnnagg_gcn_run_bf16(self.h, _bf16(X, "X"), _f32(Y, "Y"), X.shape[1], int(scheduled), _stream()))
+        else:
+            check(lib().gnnagg_gcn_run(self.h, _f32(X, "X"), _f32(Y, "Y"), X.shape[1], int(scheduled), _stream()))
         return Y
 
     def gcn_run_acc(self, X, Y, accumulate=True):
@@ -431,8 +457,12 @@ class Aggregator:
         return out
 
     def gcn_layer(self, X, W, H, AX=None, scheduled=False):
-        check(lib().gnnagg_gcn_layer(self.h, _f32(X, "X"), _f32(W, "W"), _f32(H, "H"), _f32(AX, "AX"), W.shape[0], W.shape[1], int(scheduled),
-                                     _stream()))
+        if _is_bf16(X):
+            check(lib().gnnagg_gcn_layer_bf16(self.h, _bf16(X, "X"), _f32(W, "W"), _f32(H, "H"), _f32(AX, "AX"), W.shape[0],
+                                              W.shape[1], int(scheduled), _stream()))
+        else:
+            check(lib().gnnagg_gcn_layer(self.h, _f32(X, "X"), _f32(W, "W"), _f32(H, "H"), _f32(AX, "AX"), W.shape[0], W.shape[1], int(scheduled),
+                                         _stream()))
         return H
 
     # --- GAT
@@ -489,7 +519,10 @@ class Aggregator:
         return back(tp, ns.value + 1), back(ti, self.m), back(tq, self.m)
 
     def gcn_backward(self, dY, dX):
-        check(lib().gnnagg_gcn_backward(self.h, _f32(dY, "dY"), _f32(dX, "dX"), dY.shape[1], _stream()))
+        if _is_bf16(dY):
+            check(lib().gnnagg_gcn_backward_bf16(self.h, _bf16(dY, "dY"), _f32(dX, "dX"), dY.shape[1], _stream()))
+        else:
+            check(lib().gnnagg_gcn_backward(self.h, _f32(dY, "dY"), _f32(dX, "dX"), dY.shape[1], _stream()))
         return dX
 
     def gat_backward(self, X, att, Y, dY, dX, datt, slope=0.2, w=None, den=None):

@@ -117,7 +117,8 @@ def _transposed(agg, num_src):
 
 class GCNAggregate(torch.autograd.Function):
     """Y = A X for the aggregator `at` (edge values are constants of the graph).  backward: dX = A^T dY through the
-    GPU-built transposed CSR (deterministic gather, no atomics)."""
+    GPU-built transposed CSR (deterministic gather, no atomics).  X may be float32 or bfloat16; Y is float32.  dX is
+    computed in float32 and rounded once to X's dtype."""
 
     @staticmethod
     def forward(ctx, at, X, scheduled=False):
@@ -126,7 +127,7 @@ class GCNAggregate(torch.autograd.Function):
         _check(X)
         Y = torch.empty((agg.n, X.shape[1]), device=X.device, dtype=torch.float32)
         agg.gcn_run(X, Y, bool(scheduled))
-        ctx.at, ctx.num_src = at, X.shape[0]
+        ctx.at, ctx.num_src, ctx.x_dtype = at, X.shape[0], X.dtype
         return Y
 
     @staticmethod
@@ -134,7 +135,7 @@ class GCNAggregate(torch.autograd.Function):
         agg = _transposed(_get(ctx.at), ctx.num_src)
         dX = torch.empty((ctx.num_src, dY.shape[1]), device=dY.device, dtype=torch.float32)
         agg.gcn_backward(dY.contiguous(), dX)
-        return None, dX, None
+        return None, dX.to(ctx.x_dtype), None
 
 
 class GATAggregate(torch.autograd.Function):

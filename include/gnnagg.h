@@ -253,6 +253,22 @@ int gnnagg_gcn_backward(gnnagg_aggregator *a, const float *dY, float *dX, int fe
 int gnnagg_gat_backward(gnnagg_aggregator *a, const float *X, const float *att, const float *w, const float *den,
                         const float *Y, const float *dY, float *dX, float *datt, int feat, float slope, void *stream);
 
+/* ---- GCN aggregation from bf16 features ------------------------------------------------------------------
+ * The same operations as gnnagg_gcn_run, gnnagg_gcn_layer and gnnagg_gcn_backward with the GATHERED operand (X, or dY
+ * of the backward) stored in bf16: X / dY are bf16 bit patterns, 8-byte aligned, [rows, feat] row-major.  Edge values,
+ * accumulation and every output (Y, H, AX, dX) stay fp32, outputs 16-byte aligned; feat is a multiple of 4 in
+ * [4, 1024] as for fp32.  Each bf16 value is widened exactly to fp32 on load and then summed as in the fp32 run, so
+ * the result equals the fp32 entry point run on the widened X, bit for bit for un-scheduled runs (CSR, merged view,
+ * locality slices) and up to the arbitrary RED.ADD order of scheduled runs.  Routing, the settings, profiling
+ * (gnnagg_profile_read) and the launch count are those of the fp32 entry point; gnnagg_prepare also readies the bf16
+ * kernel.  The automatic locality-slice rule sizes X from the bytes stored (2 per element); its constants were tuned
+ * on fp32 runs and are not re-tuned for bf16.  gnnagg_gcn_layer_bf16 uses the same fp32 combination as
+ * gnnagg_gcn_layer on the fp32 AX. */
+int gnnagg_gcn_run_bf16(gnnagg_aggregator *a, const uint16_t *X, float *Y, int feat, int scheduled, void *stream);
+int gnnagg_gcn_layer_bf16(gnnagg_aggregator *a, const uint16_t *X, const float *W, float *H, float *AX, int feat_in,
+                          int feat_out, int scheduled, void *stream);
+int gnnagg_gcn_backward_bf16(gnnagg_aggregator *a, const uint16_t *dY, float *dX, int feat, void *stream);
+
 /* ---- sub-graph samplers (SURVEY §8(f) rank 4) -------------------------------------------------------------
  * replaces sampleVertex (include/sample.h:131-200) and sampleVertexSampleNeighbor (:274-357).
  * d_active [num_v]: non-zero marks the seed vertices; on return it holds the 0/1 set after layer_num - 1 hops
