@@ -1160,17 +1160,29 @@ int gnnagg_prepare(gnnagg_aggregator *a, int feat, void *stream)
     return host_ptr(v, &hp);  // row-range launches (gnnagg_gcn_run_rows) cut edge ranges on the host
 }
 
-int gnnagg_gcn_run_rows(gnnagg_aggregator *a, const float *X, float *Y, int feat, int accumulate, int row_lo, int row_hi,
-                        void *stream)
+static int gcn_run_rows_impl(gnnagg_aggregator *a, GatherX X, float *Y, int feat, int accumulate, int row_lo, int row_hi,
+                             cudaStream_t st)
 {
     if (!a) return set_error(GNNAGG_ERR_ARG, "gnnagg_gcn_run_rows: NULL aggregator");
     if (row_lo < 0 || row_hi > a->n || row_lo > row_hi) return set_error(GNNAGG_ERR_ARG, "gnnagg_gcn_run_rows: bad row range");
     if (row_lo == row_hi) return GNNAGG_OK;
     View *t = a;
-    if (int rc = merged_view(a, (cudaStream_t)stream, &t)) return rc;
+    if (int rc = merged_view(a, st, &t)) return rc;
     const int *hp = nullptr;
     if (int rc = host_ptr(*t, &hp)) return rc;
-    return gcn_run_core(*t, X, Y, feat, 0, (cudaStream_t)stream, accumulate != 0, row_lo, row_hi, hp[row_lo], hp[row_hi]);
+    return gcn_run_core(*t, X, Y, feat, 0, st, accumulate != 0, row_lo, row_hi, hp[row_lo], hp[row_hi]);
+}
+
+int gnnagg_gcn_run_rows(gnnagg_aggregator *a, const float *X, float *Y, int feat, int accumulate, int row_lo, int row_hi,
+                        void *stream)
+{
+    return gcn_run_rows_impl(a, X, Y, feat, accumulate, row_lo, row_hi, (cudaStream_t)stream);
+}
+
+int gnnagg_gcn_run_rows_bf16(gnnagg_aggregator *a, const uint16_t *X, float *Y, int feat, int accumulate, int row_lo,
+                             int row_hi, void *stream)
+{
+    return gcn_run_rows_impl(a, X, Y, feat, accumulate, row_lo, row_hi, (cudaStream_t)stream);
 }
 
 int gnnagg_gcn_run(gnnagg_aggregator *a, const float *X, float *Y, int feat, int scheduled, void *stream)
@@ -1184,6 +1196,11 @@ int gnnagg_gcn_run_bf16(gnnagg_aggregator *a, const uint16_t *X, float *Y, int f
 }
 
 int gnnagg_gcn_run_acc(gnnagg_aggregator *a, const float *X, float *Y, int feat, int accumulate, void *stream)
+{
+    return gcn_run_impl(a, X, Y, feat, 0, (cudaStream_t)stream, true, accumulate != 0);
+}
+
+int gnnagg_gcn_run_acc_bf16(gnnagg_aggregator *a, const uint16_t *X, float *Y, int feat, int accumulate, void *stream)
 {
     return gcn_run_impl(a, X, Y, feat, 0, (cudaStream_t)stream, true, accumulate != 0);
 }

@@ -133,40 +133,43 @@ __global__ void __launch_bounds__(32) halo_consumed_kernel(PeerTable peers, int 
 // into what three aggregation CTAs (3 x 256 threads x 80 registers) leave free on an SM; the first version (256 threads,
 // 8 loads in flight per thread, 2 CTAs per SM) displaced one aggregation CTA per SM for as long as the exchange ran.
 // Posted writes need no latency hiding; U loads per thread cover the local gather latency.
-template <int U, bool PREFETCH>
-__global__ void __launch_bounds__(128, 16) halo_push_kernel(const float4 *__restrict__ X, const int *__restrict__ rows,
-                                                            float4 *__restrict__ dst, int64_t count4, int F4, int f4_shift,
+// The rows are copied in units of T, whatever they hold: float4 for fp32 rows and for bf16 rows of a width that is a
+// multiple of 8; uint2 for bf16 rows of a width that is 4 mod 8 (F = 100: 200 bytes, 8-byte aligned only).  FU = units
+// per row, fu_shift = log2(FU) when FU is a power of two (else -1), units = rows x FU.
+template <typename T, int U, bool PREFETCH>
+__global__ void __launch_bounds__(128, 16) halo_push_kernel(const T *__restrict__ X, const int *__restrict__ rows,
+                                                            T *__restrict__ dst, int64_t units, int FU, int fu_shift,
                                                             uint32_t *done_cnt, uint32_t *arrived_flag, uint32_t value)
 {
     const int64_t stride = (int64_t)gridDim.x * 128 * U;
-    for (int64_t base = (int64_t)blockIdx.x * 128 * U + threadIdx.x; base < count4; base += stride) {
+    for (int64_t base = (int64_t)blockIdx.x * 128 * U + threadIdx.x; base < units; base += stride) {
         if (PREFETCH) {
             // the rows of the NEXT iteration are pulled into L2 now: prefetches hold no registers, so the kernel has twice
             // its load depth in flight where the memory system is busy with the aggregation's gathers
 #pragma unroll
             for (int u = 0; u < U; ++u) {
                 const int64_t e = base + stride + (int64_t)u * 128;
-                if (e < count4 && (e & 7) == 0) {  // one prefetch per 128-byte line
-                    const int64_t r = (f4_shift >= 0) ? (e >> f4_shift) : (e / F4);
-                    const int c = (int)(e - r * F4);
-                    asm volatile("prefetch.global.L2 [%0];" ::"l"(X + (int64_t)__ldg(rows + r) * F4 + c));
+                if (e < units && (e & (int64_t)(128 / sizeof(T) - 1)) == 0) {  // one prefetch per 128-byte line
+                    const int64_t r = (fu_shift >= 0) ? (e >> fu_shift) : (e / FU);
+                    const int c = (int)(e - r * FU);
+                    asm volatile("prefetch.global.L2 [%0];" ::"l"(X + (int64_t)__ldg(rows + r) * FU + c));
                 }
             }
         }
-        float4 v[U];
+        T v[U];
 #pragma unroll
         for (int u = 0; u < U; ++u) {
             const int64_t e = base + (int64_t)u * 128;
-            if (e < count4) {
-                const int64_t r = (f4_shift >= 0) ? (e >> f4_shift) : (e / F4);
-                const int c = (int)(e - r * F4);
-                v[u] = __ldg(X + (int64_t)__ldg(rows + r) * F4 + c);
+            if (e < units) {
+                const int64_t r = (fu_shift >= 0) ? (e >> fu_shift) : (e / FU);
+                const int c = (int)(e - r * FU);
+                v[u] = __ldg(X + (int64_t)__ldg(rows + r) * FU + c);
             }
         }
 #pragma unroll
         for (int u = 0; u < U; ++u) {
             const int64_t e = base + (int64_t)u * 128;
-            if (e < count4) dst[e] = v[u];
+            if (e < units) dst[e] = v[u];
         }
     }
     // every thread's stores are ordered before this CTA's count, the count before the flag (system scope)
@@ -595,8 +598,9 @@ int gnnagg_dist_create_rank(int rank, int world, const int64_t *shard_bounds, in
         if (cudaFuncGetAttributes(&attr, halo_begin_kernel) != cudaSuccess) cudaGetLastError();
         if (cudaFuncGetAttributes(&attr, halo_wait_kernel) != cudaSuccess) cudaGetLastError();
         if (cudaFuncGetAttributes(&attr, halo_consumed_kernel) != cudaSuccess) cudaGetLastError();
-        if (cudaFuncGetAttributes(&attr, halo_push_kernel<4, false>) != cudaSuccess) cudaGetLastError();
-        if (cudaFuncGetAttributes(&attr, halo_push_kernel<4, true>) != cudaSuccess) cudaGetLastError();
+        if (cudaFuncGetAttributes(&attr, halo_push_kernel<float4, 4, false>) != cudaSuccess) cudaGetLastError();
+        if (cudaFuncGetAttributes(&attr, halo_push_kernel<uint2, 4, false>) != cudaSuccess) cudaGetLastError();  // bf16, F = 4 mod 8
+        if (cudaFuncGetAttributes(&attr, halo_push_kernel<float4, 4, true>) != cudaSuccess) cudaGetLastError();
         if (const char *env = getenv("GNNAGG_PUSH_PREFETCH")) d->push_prefetch = atoi(env) != 0;
         if (cudaFuncGetAttributes(&attr, halo_push_heavy_kernel<8>) != cudaSuccess) cudaGetLastError();
         if (const char *env = getenv("GNNAGG_PUSH_HEAVY")) d->push_heavy = atoi(env);
@@ -1093,9 +1097,24 @@ int64_t gnnagg_dist_launch_count(const gnnagg_dist *d)
 // receive buffer of the previous step (kernels-only timing).
 // host_out != NULL: the LAST stage runs in kHostChunks row chunks; chunk c is aggregated (and combined) on `st` while
 // the finished rows of chunk c-1 travel to host_out on a second stream (Y / H then are device staging).
+// bf16: the shards and receive slots hold bf16 rows of stride feat_in (every address into them is computed in bytes);
+// Y, AX and H stay fp32.
 constexpr int kHostChunks = 4;
 
-static int dist_run(gnnagg_dist *d, int buf, float *Y, const float *W, float *H, int feat_in, int feat_out, int flags,
+static int stage_run_acc(gnnagg_aggregator *a, bool bf16, const char *xs, float *Y, int feat, int accumulate, cudaStream_t st)
+{
+    return bf16 ? gnnagg_gcn_run_acc_bf16(a, reinterpret_cast<const uint16_t *>(xs), Y, feat, accumulate, st)
+                : gnnagg_gcn_run_acc(a, reinterpret_cast<const float *>(xs), Y, feat, accumulate, st);
+}
+
+static int stage_run_rows(gnnagg_aggregator *a, bool bf16, const char *xs, float *Y, int feat, int accumulate, int r0, int r1,
+                          cudaStream_t st)
+{
+    return bf16 ? gnnagg_gcn_run_rows_bf16(a, reinterpret_cast<const uint16_t *>(xs), Y, feat, accumulate, r0, r1, st)
+                : gnnagg_gcn_run_rows(a, reinterpret_cast<const float *>(xs), Y, feat, accumulate, r0, r1, st);
+}
+
+static int dist_run(gnnagg_dist *d, int buf, bool bf16, float *Y, const float *W, float *H, int feat_in, int feat_out, int flags,
                     cudaStream_t st, float *host_out = nullptr)
 {
     if (!d || (!Y && d->rows > 0) || buf < 0 || buf > 1) return set_error(GNNAGG_ERR_ARG, "gnnagg_dist_gcn_run: bad argument");
@@ -1112,7 +1131,8 @@ static int dist_run(gnnagg_dist *d, int buf, float *Y, const float *W, float *H,
     // kernels spin on this rank's flags would never return)
     if (d->prepared_feat != feat_in)
         if (int rc = gnnagg_dist_prepare(d, feat_in, st)) return rc;
-    const float *xs = reinterpret_cast<const float *>(d->base + d->off_x[buf]);  // shard rows, then the receive slots
+    const char *xs = d->base + d->off_x[buf];  // shard rows, then the receive slots
+    const size_t row_bytes = (size_t)feat_in * (bf16 ? 2 : 4);
     HaloFlags *mine = flags_of(d->base);
     uint32_t epoch = d->epoch;
     // arrived[] counts completed pushes: round c of epoch e raises it to (e - 1) * rounds + c + 1
@@ -1127,45 +1147,52 @@ static int dist_run(gnnagg_dist *d, int buf, float *Y, const float *W, float *H,
         DT_TRY(cudaEventRecord(d->ev_sig, st));
         DT_TRY(cudaStreamWaitEvent(d->comm, d->ev_sig, 0));
         if (d->prof) DT_TRY(cudaEventRecord(d->t_c0, d->comm));
-        const int F4 = feat_in / 4;
+        // copy units of the push: 16 bytes, or 8 for bf16 rows of a width that is 4 mod 8 (8-byte aligned only)
+        const bool narrow = bf16 && (feat_in & 7);
+        const int FU = (int)(row_bytes / (narrow ? sizeof(uint2) : sizeof(float4)));
         int shift = -1;
         for (int s = 0; s < 16; ++s)
-            if ((1 << s) == F4) shift = s;
+            if ((1 << s) == FU) shift = s;
         for (int c = 0; c < d->rounds; ++c) {
             for (int k = 0; k < Wd - 1; ++k) {
                 const int q = (d->rank - 1 - k + 2 * Wd) % Wd;  // receiver q takes this owner as its k-th
-                const int64_t count4 = (int64_t)d->send_cnt[q][c] * F4;
+                const int64_t units = (int64_t)d->send_cnt[q][c] * FU;
                 // one light CTA per SM (two when the round is large) keeps the link busy; ranks sharing a device (tests) split that
-                int64_t grid = (count4 + 128 * 4 - 1) / (128 * 4);
+                int64_t grid = (units + 128 * 4 - 1) / (128 * 4);
                 const int64_t cap = d->same_device_ranks > 1 ? std::max(4, d->sm_count / (2 * d->same_device_ranks)) : 2 * d->sm_count;
                 grid = grid < 1 ? 1 : (grid > cap ? cap : grid);  // an empty push still raises the flag
-                float *dst = reinterpret_cast<float *>(d->peer_base[q] + d->peer_off_x[q][buf]) +
-                             ((size_t)d->peer_rows[q] + (size_t)d->peer_slot[q][c]) * feat_in;
+                char *dst = d->peer_base[q] + d->peer_off_x[q][buf] + ((size_t)d->peer_rows[q] + (size_t)d->peer_slot[q][c]) * row_bytes;
                 const int *list = d->send_rows[q] ? d->send_rows[q] + d->send_off[q][c] : nullptr;
                 uint32_t *flag = &flags_of(d->peer_base[q])->arrived[d->rank];
-                if (d->push_tma && feat_in * 4 <= kPushBatchBytes) {
+                // bf16 steps always take the default kernel: the GNNAGG_PUSH_* experiments are fp32 only
+                if (!bf16 && d->push_tma && feat_in * 4 <= kPushBatchBytes) {
                     int rpb = kPushBatchBytes / (feat_in * 4);
                     rpb = rpb > 32 ? 32 : rpb;
                     int64_t g2 = (d->send_cnt[q][c] + rpb - 1) / rpb;
                     const int64_t cap2 = d->same_device_ranks > 1 ? std::max(4, d->sm_count / (2 * d->same_device_ranks)) : 2 * d->sm_count;
                     g2 = g2 < 1 ? 1 : (g2 > cap2 ? cap2 : g2);
                     halo_push_tma_kernel<<<(unsigned)g2, 32, kPushBufs * kPushBatchBytes, d->comm>>>(
-                        xs, list, dst, d->send_cnt[q][c], feat_in, rpb, &mine->push_cnt[q], flag, flag_base + (uint32_t)c + 1u);
-                } else if (d->push_heavy) {
-                    int64_t gh = (count4 + 256 * 8 - 1) / (256 * 8);
+                        reinterpret_cast<const float *>(xs), list, reinterpret_cast<float *>(dst), d->send_cnt[q][c], feat_in, rpb,
+                        &mine->push_cnt[q], flag, flag_base + (uint32_t)c + 1u);
+                } else if (!bf16 && d->push_heavy) {
+                    int64_t gh = (units + 256 * 8 - 1) / (256 * 8);
                     const int64_t caph = d->same_device_ranks > 1 ? std::max(4, d->sm_count / (2 * d->same_device_ranks)) : (int64_t)d->push_heavy * d->sm_count;
                     gh = gh < 1 ? 1 : (gh > caph ? caph : gh);
                     halo_push_heavy_kernel<8><<<(unsigned)gh, 256, 0, d->comm>>>(reinterpret_cast<const float4 *>(xs), list,
-                                                                               reinterpret_cast<float4 *>(dst), count4, F4, shift,
+                                                                               reinterpret_cast<float4 *>(dst), units, FU, shift,
                                                                                &mine->push_cnt[q], flag, flag_base + (uint32_t)c + 1u);
-                } else if (d->push_prefetch) {
-                    halo_push_kernel<4, true><<<(unsigned)grid, 128, 0, d->comm>>>(reinterpret_cast<const float4 *>(xs), list,
-                                                                                 reinterpret_cast<float4 *>(dst), count4, F4, shift,
-                                                                                 &mine->push_cnt[q], flag, flag_base + (uint32_t)c + 1u);
+                } else if (!bf16 && d->push_prefetch) {
+                    halo_push_kernel<float4, 4, true><<<(unsigned)grid, 128, 0, d->comm>>>(
+                        reinterpret_cast<const float4 *>(xs), list, reinterpret_cast<float4 *>(dst), units, FU, shift, &mine->push_cnt[q],
+                        flag, flag_base + (uint32_t)c + 1u);
+                } else if (narrow) {
+                    halo_push_kernel<uint2, 4, false><<<(unsigned)grid, 128, 0, d->comm>>>(
+                        reinterpret_cast<const uint2 *>(xs), list, reinterpret_cast<uint2 *>(dst), units, FU, shift, &mine->push_cnt[q],
+                        flag, flag_base + (uint32_t)c + 1u);
                 } else {
-                    halo_push_kernel<4, false><<<(unsigned)grid, 128, 0, d->comm>>>(reinterpret_cast<const float4 *>(xs), list,
-                                                                                  reinterpret_cast<float4 *>(dst), count4, F4, shift,
-                                                                                  &mine->push_cnt[q], flag, flag_base + (uint32_t)c + 1u);
+                    halo_push_kernel<float4, 4, false><<<(unsigned)grid, 128, 0, d->comm>>>(
+                        reinterpret_cast<const float4 *>(xs), list, reinterpret_cast<float4 *>(dst), units, FU, shift, &mine->push_cnt[q],
+                        flag, flag_base + (uint32_t)c + 1u);
                 }
                 DT_TRY(cudaPeekAtLastError());
                 ++d->launches;
@@ -1194,7 +1221,7 @@ static int dist_run(gnnagg_dist *d, int buf, float *Y, const float *W, float *H,
             ++d->launches;
         }
         if (!by_rounds && !by_chunks) {
-            if (int rc = gnnagg_gcn_run_acc(d->stage[s], xs, agg_out, feat_in, s > 0, st)) return rc;
+            if (int rc = stage_run_acc(d->stage[s], bf16, xs, agg_out, feat_in, s > 0, st)) return rc;
             if (s == 0 && d->prof) DT_TRY(cudaEventRecord(d->t_m1, st));
             continue;
         }
@@ -1210,7 +1237,7 @@ static int dist_run(gnnagg_dist *d, int buf, float *Y, const float *W, float *H,
                 ++d->launches;
             }
             if (r1 <= r0) continue;
-            if (int rc = gnnagg_gcn_run_rows(d->stage[s], xs, agg_out, feat_in, s > 0, r0, r1, st)) return rc;
+            if (int rc = stage_run_rows(d->stage[s], bf16, xs, agg_out, feat_in, s > 0, r0, r1, st)) return rc;
             if (!host_out) continue;
             if (W) {
                 if (int rc = gnnagg_dense_nn(d->ax + (size_t)r0 * feat_in, W, H + (size_t)r0 * feat_out, r1 - r0, feat_out, feat_in, st))
@@ -1255,17 +1282,34 @@ static int dist_run(gnnagg_dist *d, int buf, float *Y, const float *W, float *H,
 
 int gnnagg_dist_gcn_run(gnnagg_dist *d, int buf, float *Y, int feat, int flags, void *stream)
 {
-    return dist_run(d, buf, Y, nullptr, nullptr, feat, feat, flags, (cudaStream_t)stream);
+    return dist_run(d, buf, false, Y, nullptr, nullptr, feat, feat, flags, (cudaStream_t)stream);
+}
+
+int gnnagg_dist_gcn_run_bf16(gnnagg_dist *d, int buf, float *Y, int feat, int flags, void *stream)
+{
+    return dist_run(d, buf, true, Y, nullptr, nullptr, feat, feat, flags, (cudaStream_t)stream);
+}
+
+static int dist_layer(gnnagg_dist *d, int buf, bool bf16, const float *W, float *H, int feat_in, int feat_out, int flags,
+                      void *stream)
+{
+    if (!W || (!H && d && d->rows > 0)) return set_error(GNNAGG_ERR_ARG, "gnnagg_dist_gcn_layer: NULL argument");
+    return dist_run(d, buf, bf16, H, W, H, feat_in, feat_out, flags, (cudaStream_t)stream);
 }
 
 int gnnagg_dist_gcn_layer(gnnagg_dist *d, int buf, const float *W, float *H, int feat_in, int feat_out, int flags, void *stream)
 {
-    if (!W || (!H && d && d->rows > 0)) return set_error(GNNAGG_ERR_ARG, "gnnagg_dist_gcn_layer: NULL argument");
-    return dist_run(d, buf, H, W, H, feat_in, feat_out, flags, (cudaStream_t)stream);
+    return dist_layer(d, buf, false, W, H, feat_in, feat_out, flags, stream);
 }
 
-int gnnagg_dist_gcn_layer_host(gnnagg_dist *d, int buf, const float *h_X, const float *h_W, float *h_out, int feat_in,
-                               int feat_out, void *stream)
+int gnnagg_dist_gcn_layer_bf16(gnnagg_dist *d, int buf, const float *W, float *H, int feat_in, int feat_out, int flags,
+                               void *stream)
+{
+    return dist_layer(d, buf, true, W, H, feat_in, feat_out, flags, stream);
+}
+
+static int dist_layer_host(gnnagg_dist *d, int buf, bool bf16, const void *h_X, const float *h_W, float *h_out, int feat_in,
+                           int feat_out, void *stream)
 {
     if (!d || (d->rows > 0 && (!h_X || !h_out)) || buf < 0 || buf > 1)
         return set_error(GNNAGG_ERR_ARG, "gnnagg_dist_gcn_layer_host: bad argument");
@@ -1292,12 +1336,24 @@ int gnnagg_dist_gcn_layer_host(gnnagg_dist *d, int buf, const float *h_X, const 
     }
     DT_TRY(cudaEventRecord(d->copies_done, d->copy_stream));  // so that the wait below is defined when no chunk copy is issued
     if (d->rows > 0)
-        DT_TRY(cudaMemcpyAsync(d->base + d->off_x[buf], h_X, (size_t)d->rows * feat_in * sizeof(float), cudaMemcpyHostToDevice, st));
+        DT_TRY(cudaMemcpyAsync(d->base + d->off_x[buf], h_X, (size_t)d->rows * feat_in * (bf16 ? 2 : 4), cudaMemcpyHostToDevice, st));
     if (h_W) DT_TRY(cudaMemcpyAsync(d->st_w, h_W, (size_t)feat_in * feat_out * sizeof(float), cudaMemcpyHostToDevice, st));
-    if (int rc = dist_run(d, buf, d->st_out, h_W ? d->st_w : nullptr, d->st_out, feat_in, feat_out, 0, st, h_out)) return rc;
+    if (int rc = dist_run(d, buf, bf16, d->st_out, h_W ? d->st_w : nullptr, d->st_out, feat_in, feat_out, 0, st, h_out)) return rc;
     DT_TRY(cudaStreamWaitEvent(st, d->copies_done, 0));
     DT_TRY(cudaStreamSynchronize(st));
     return GNNAGG_OK;
+}
+
+int gnnagg_dist_gcn_layer_host(gnnagg_dist *d, int buf, const float *h_X, const float *h_W, float *h_out, int feat_in,
+                               int feat_out, void *stream)
+{
+    return dist_layer_host(d, buf, false, h_X, h_W, h_out, feat_in, feat_out, stream);
+}
+
+int gnnagg_dist_gcn_layer_host_bf16(gnnagg_dist *d, int buf, const uint16_t *h_X, const float *h_W, float *h_out, int feat_in,
+                                    int feat_out, void *stream)
+{
+    return dist_layer_host(d, buf, true, h_X, h_W, h_out, feat_in, feat_out, stream);
 }
 
 }  // extern "C"

@@ -72,6 +72,8 @@ _SIGS = {
     "gnnagg_gcn_run_bf16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "gnnagg_gcn_run_rows": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "gnnagg_gcn_run_acc": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
+    "gnnagg_gcn_run_rows_bf16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "gnnagg_gcn_run_acc_bf16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "gnnagg_gcn_run_edgewise": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "gnnagg_csr2edgelist": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "gnnagg_gcn_layer": (C.c_int, [C.c_void_p] * 5 + [C.c_int, C.c_int, C.c_int, C.c_void_p]),
@@ -123,6 +125,10 @@ _SIGS = {
     "gnnagg_dist_gcn_run": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "gnnagg_dist_gcn_layer": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "gnnagg_dist_gcn_layer_host": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
+    "gnnagg_dist_gcn_run_bf16": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
+    "gnnagg_dist_gcn_layer_bf16": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "gnnagg_dist_gcn_layer_host_bf16": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
+                                                  C.c_void_p]),
     "gnnagg_dist_info": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(C.c_int),
                                    C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "gnnagg_dist_connect_local": (C.c_int, [C.POINTER(C.c_void_p), C.c_int]),
@@ -278,17 +284,17 @@ def _f32(t, name, cuda=True):
     return C.c_void_p(t.data_ptr())
 
 
-def _bf16(t, name):
-    """device bfloat16 operand (the gathered X / dY of the bf16 GCN entry points); numpy has no bf16, so there is
-    no host path"""
+def _bf16(t, name, cuda=True):
+    """bfloat16 torch operand (the gathered X / dY of the bf16 GCN entry points, or the host X shard of
+    gnnagg_dist_gcn_layer_host_bf16 with cuda=False); numpy has no bf16, so numpy arrays are not accepted"""
     import torch
 
-    if t.dtype != torch.bfloat16:
+    if isinstance(t, np.ndarray) or t.dtype != torch.bfloat16:
         raise GnnaggError("%s: expected bfloat16, got %s" % (name, t.dtype))
     if not t.is_contiguous():
         raise GnnaggError("%s: expected a contiguous row-major tensor (got strides %s)" % (name, tuple(t.stride())))
-    if not t.is_cuda:
-        raise GnnaggError("%s: expected a CUDA tensor" % name)
+    if bool(t.is_cuda) != bool(cuda):
+        raise GnnaggError("%s: expected a %s tensor" % (name, "CUDA" if cuda else "host"))
     return C.c_void_p(t.data_ptr())
 
 
@@ -440,12 +446,19 @@ class Aggregator:
         return Y
 
     def gcn_run_acc(self, X, Y, accumulate=True):
-        check(lib().gnnagg_gcn_run_acc(self.h, _f32(X, "X"), _f32(Y, "Y"), X.shape[1], int(accumulate), _stream()))
+        if _is_bf16(X):
+            check(lib().gnnagg_gcn_run_acc_bf16(self.h, _bf16(X, "X"), _f32(Y, "Y"), X.shape[1], int(accumulate), _stream()))
+        else:
+            check(lib().gnnagg_gcn_run_acc(self.h, _f32(X, "X"), _f32(Y, "Y"), X.shape[1], int(accumulate), _stream()))
         return Y
 
     def gcn_run_rows(self, X, Y, row_lo, row_hi, accumulate=False):
-        check(lib().gnnagg_gcn_run_rows(self.h, _f32(X, "X"), _f32(Y, "Y"), X.shape[1], int(accumulate), int(row_lo), int(row_hi),
-                                        _stream()))
+        if _is_bf16(X):
+            check(lib().gnnagg_gcn_run_rows_bf16(self.h, _bf16(X, "X"), _f32(Y, "Y"), X.shape[1], int(accumulate), int(row_lo),
+                                                 int(row_hi), _stream()))
+        else:
+            check(lib().gnnagg_gcn_run_rows(self.h, _f32(X, "X"), _f32(Y, "Y"), X.shape[1], int(accumulate), int(row_lo), int(row_hi),
+                                            _stream()))
         return Y
 
     def gcn_run_edgewise(self, X, Y):

@@ -314,11 +314,12 @@ class PipelinedPrunedHalo:
 # handles) at set-up, and for the barriers of the teardown.
 # ------------------------------------------------------------------------------------------------
 class _DeviceMemory:
-    """a library-owned device buffer exposed through __cuda_array_interface__ (zero-copy torch view)"""
+    """a library-owned device buffer exposed through __cuda_array_interface__ (zero-copy torch view).  The interface
+    has no bf16 typestr: a bf16 view is taken as "<i2" and reinterpreted with .view(torch.bfloat16)."""
 
-    def __init__(self, ptr, shape, owner):
+    def __init__(self, ptr, shape, owner, typestr="<f4"):
         self.owner = owner
-        self.__cuda_array_interface__ = {"shape": tuple(int(s) for s in shape), "typestr": "<f4", "data": (int(ptr), False),
+        self.__cuda_array_interface__ = {"shape": tuple(int(s) for s in shape), "typestr": typestr, "data": (int(ptr), False),
                                          "version": 3, "strides": None}
 
 
@@ -386,39 +387,66 @@ class PeerHalo:
         self.num_send = sum(self.send_counts)
         self.referenced_fraction = (self.num_recv + 0.0) / max(1, self.bounds[-1])
 
-    def x(self, buf=0, feat=None):
-        """torch view [rows, feat] of peer-visible shard buffer `buf` (write X here, or let a layer write H here)"""
+    def x(self, buf=0, feat=None, dtype=None):
+        """torch view [rows, feat] of peer-visible shard buffer `buf` (write X here, or let a layer write H here).
+        dtype torch.float32 (default) or torch.bfloat16: a bf16 shard of the same width takes half of the buffer; steps
+        on it pass dtype=torch.bfloat16 too"""
         import torch
 
         from . import lib
 
+        dtype = torch.float32 if dtype is None else dtype
+        if dtype not in (torch.float32, torch.bfloat16):
+            raise ValueError("PeerHalo.x: dtype must be torch.float32 or torch.bfloat16, got %s" % dtype)
         feat = self.feat_cap if feat is None else feat
         p = lib().gnnagg_dist_x(self.h, int(buf))
         if self.rows == 0:
-            return torch.empty((0, feat), device=self.device)
+            return torch.empty((0, feat), device=self.device, dtype=dtype)
+        if dtype == torch.bfloat16:
+            return torch.as_tensor(_DeviceMemory(p, (self.rows, feat), self, "<i2"), device=self.device).view(torch.bfloat16)
         return torch.as_tensor(_DeviceMemory(p, (self.rows, feat), self), device=self.device)
 
-    def gcn_run(self, Y, buf=0, feat=None, exchange=True):
+    @staticmethod
+    def _is_bf16(dtype):
+        import torch
+
+        if dtype is None or dtype == torch.float32:
+            return False
+        if dtype == torch.bfloat16:
+            return True
+        raise ValueError("the shard dtype must be torch.float32 or torch.bfloat16, got %s" % dtype)
+
+    def gcn_run(self, Y, buf=0, feat=None, exchange=True, dtype=None):
+        """Y = A_block X with X = shard buffer `buf` of every rank, stored as `dtype` (float32 or bfloat16; Y is float32)"""
         from . import DIST_NO_EXCHANGE, _f32, _stream, check, lib
 
         feat = Y.shape[1] if feat is None else feat
-        check(lib().gnnagg_dist_gcn_run(self.h, int(buf), _f32(Y, "Y"), int(feat), 0 if exchange else DIST_NO_EXCHANGE, _stream()))
+        run = lib().gnnagg_dist_gcn_run_bf16 if self._is_bf16(dtype) else lib().gnnagg_dist_gcn_run
+        check(run(self.h, int(buf), _f32(Y, "Y"), int(feat), 0 if exchange else DIST_NO_EXCHANGE, _stream()))
         return Y
 
-    def gcn_layer(self, W, H, buf=0, exchange=True):
+    def gcn_layer(self, W, H, buf=0, exchange=True, dtype=None):
+        """H = (A_block X) W with X = shard buffer `buf` stored as `dtype` (float32 or bfloat16; W, H are float32)"""
         from . import DIST_NO_EXCHANGE, _f32, _stream, check, lib
 
-        check(lib().gnnagg_dist_gcn_layer(self.h, int(buf), _f32(W, "W"), _f32(H, "H"), W.shape[0], W.shape[1],
-                                          0 if exchange else DIST_NO_EXCHANGE, _stream()))
+        run = lib().gnnagg_dist_gcn_layer_bf16 if self._is_bf16(dtype) else lib().gnnagg_dist_gcn_layer
+        check(run(self.h, int(buf), _f32(W, "W"), _f32(H, "H"), W.shape[0], W.shape[1], 0 if exchange else DIST_NO_EXCHANGE,
+                  _stream()))
         return H
 
     def gcn_layer_host(self, hX, hW, hH, buf=0):
-        """pinned host X shard (and W) -> host H (or A*X when hW is None); copies inside, synchronises the stream"""
-        from . import _f32, _stream, check, lib
+        """pinned host X shard (float32 or bfloat16) and W -> host H (or A*X when hW is None), float32; copies inside,
+        synchronises the stream"""
+        from . import _bf16, _f32, _is_bf16, _stream, check, lib
 
         fin = hX.shape[1]
-        check(lib().gnnagg_dist_gcn_layer_host(self.h, int(buf), _f32(hX, "hX", cuda=False), _f32(hW, "hW", cuda=False),
-                                               _f32(hH, "hH", cuda=False), fin, fin if hW is None else hW.shape[1], _stream()))
+        fout = fin if hW is None else hW.shape[1]
+        if _is_bf16(hX):
+            check(lib().gnnagg_dist_gcn_layer_host_bf16(self.h, int(buf), _bf16(hX, "hX", cuda=False), _f32(hW, "hW", cuda=False),
+                                                        _f32(hH, "hH", cuda=False), fin, fout, _stream()))
+        else:
+            check(lib().gnnagg_dist_gcn_layer_host(self.h, int(buf), _f32(hX, "hX", cuda=False), _f32(hW, "hW", cuda=False),
+                                                   _f32(hH, "hH", cuda=False), fin, fout, _stream()))
         return hH
 
     def profile(self, on=True):

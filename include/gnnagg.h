@@ -268,6 +268,10 @@ int gnnagg_gcn_run_bf16(gnnagg_aggregator *a, const uint16_t *X, float *Y, int f
 int gnnagg_gcn_layer_bf16(gnnagg_aggregator *a, const uint16_t *X, const float *W, float *H, float *AX, int feat_in,
                           int feat_out, int scheduled, void *stream);
 int gnnagg_gcn_backward_bf16(gnnagg_aggregator *a, const uint16_t *dY, float *dX, int feat, void *stream);
+/* bf16 forms of gnnagg_gcn_run_acc and gnnagg_gcn_run_rows (the stages of the multi-GPU step), same contract */
+int gnnagg_gcn_run_acc_bf16(gnnagg_aggregator *a, const uint16_t *X, float *Y, int feat, int accumulate, void *stream);
+int gnnagg_gcn_run_rows_bf16(gnnagg_aggregator *a, const uint16_t *X, float *Y, int feat, int accumulate, int row_lo,
+                             int row_hi, void *stream);
 
 /* ---- sub-graph samplers (SURVEY §8(f) rank 4) -------------------------------------------------------------
  * replaces sampleVertex (include/sample.h:131-200) and sampleVertexSampleNeighbor (:274-357).
@@ -318,7 +322,8 @@ int gnnagg_validate_reordered(const float *d_ref, const float *d_ans, const int 
  *                                whatever the caller has (MPI, torch.distributed, a file), gnnagg_dist_connect
  *                                (cudaIpc mapping; every owner copies the lists of rows its peers want, once)
  *   4. steps    write the X shard into gnnagg_dist_x(d, buf) on `stream`, then gnnagg_dist_gcn_run / _gcn_layer.
- *               Two shard buffers: a layer may write the next layer's input into the other one.
+ *               Two shard buffers: a layer may write the next layer's input into the other one.  A shard stored in
+ *               bf16 goes through the _bf16 forms of the steps (below): half the halo bytes, fp32 outputs.
  *   5. teardown all ranks idle -> gnnagg_dist_disconnect on every rank -> (barrier) -> gnnagg_dist_destroy
  * A step: every OWNER pushes the rows each peer wants from its shard straight into that peer's receive slots with
  * 128-bit stores over NVLink (local gathers, posted remote writes, contiguous destination; owner p serves receivers
@@ -364,6 +369,18 @@ int gnnagg_dist_gcn_layer(gnnagg_dist *d, int buf, const float *W, float *H, int
  * memory makes the copies asynchronous.  h_W NULL: aggregation only (h_out is [rows, feat_in]). */
 int gnnagg_dist_gcn_layer_host(gnnagg_dist *d, int buf, const float *h_X, const float *h_W, float *h_out, int feat_in,
                                int feat_out, void *stream);
+/* the three steps with the shard stored in bf16: gnnagg_dist_x(d, buf) (or h_X) holds bf16 bit patterns, row stride
+ * `feat` (a multiple of 4, at most feat_cap), so a shard takes half of the buffer and the halo pushes -- and the H2D copy
+ * of the host variant -- move half the bytes.  The stages gather with gnnagg_gcn_run_acc_bf16 / _rows_bf16; edge values,
+ * sums, Y, AX, the combination and H stay fp32 (as gnnagg_gcn_layer_bf16), and the result equals the fp32 step on the
+ * widened X bit for bit.  Launches, gnnagg_dist_profile_read and gnnagg_dist_prepare are those of the fp32 step; the
+ * push is always the default register kernel (the GNNAGG_PUSH_* experiments apply to fp32 steps only).  Every rank of a
+ * step must use the same dtype, buf and feat. */
+int gnnagg_dist_gcn_run_bf16(gnnagg_dist *d, int buf, float *Y, int feat, int flags, void *stream);
+int gnnagg_dist_gcn_layer_bf16(gnnagg_dist *d, int buf, const float *W, float *H, int feat_in, int feat_out, int flags,
+                               void *stream);
+int gnnagg_dist_gcn_layer_host_bf16(gnnagg_dist *d, int buf, const uint16_t *h_X, const float *h_W, float *h_out,
+                                    int feat_in, int feat_out, void *stream);
 /* distinct remote source rows this rank receives per step (in total / per owner), stages and their edge counts,
  * rows this rank pushes to every peer (after connect); any pointer may be NULL */
 int gnnagg_dist_info(const gnnagg_dist *d, int64_t *num_recv, int64_t *recv_counts /* [world] */, int *num_stages,
