@@ -506,14 +506,22 @@ __global__ void __launch_bounds__(kCtaThreads, (WE < 512) ? 4 : 3) agg_kernel(co
                 }
                 wout = wgt;
             } else if (MODE == kModeGATBWD2 && row_end - e >= U) {
+                // the batch is summed on its own, then added to the row: the duplicate edges of a (u, v) pair give the
+                // row identical terms alpha dY[v] and ds, whose rounding errors add up along one fp32 chain instead of
+                // cancelling -- EB of them (512) exceed the parity gate, EB / U + U additions stay well inside it
                 const unsigned m = vmask();
+                float4 b0 = make_float4(0.f, 0.f, 0.f, 0.f), b1 = b0;
+                float bden = 0.f;
 #pragma unroll
                 for (int u = 0; u < U; ++u) {
-                    den += __shfl_sync(m, ds_lane, u, LPR);
+                    bden += __shfl_sync(m, ds_lane, u, LPR);
                     const float wu = __shfl_sync(m, a_src, u, LPR);
-                    fma4(acc0, wu, v0[u]);
-                    if (NV > 1) fma4(acc1, wu, v1[u]);
+                    fma4(b0, wu, v0[u]);
+                    if (NV > 1) fma4(b1, wu, v1[u]);
                 }
+                den += bden;
+                acc0 = add4(acc0, b0);
+                if (NV > 1) acc1 = add4(acc1, b1);
             } else if (!mode_gat_like(MODE) && row_end - e >= U) {
                 // no row ends inside the batch: straight FMA chain (per-edge outputs: the dot products, all of row `row`)
 #pragma unroll

@@ -1233,6 +1233,7 @@ int gnnagg_gcn_layer_bf16(gnnagg_aggregator *a, const uint16_t *X, const float *
 int gnnagg_mlp_run(gnnagg_aggregator *a, const float *X, const float *W, float *Y, int feat, int scheduled,
                    void *stream)
 {
+    if (int rc = check_feat(feat)) return rc;  // the walk gathers P in float4: F % 4 != 0 would misalign its rows
     if (a && a->n == 0) return GNNAGG_OK;
     if (!a || !X || !W || !Y) return set_error(GNNAGG_ERR_ARG, "gnnagg_mlp_run: NULL argument");
     if (!aligned16(X) || !aligned16(Y)) return set_error(GNNAGG_ERR_ARG, "X and Y must be 16-byte aligned");
@@ -1240,7 +1241,7 @@ int gnnagg_mlp_run(gnnagg_aggregator *a, const float *X, const float *W, float *
     if (int rc = a->ax.ensure((size_t)a->n * feat)) return rc;
     PROF_RECORD(a, 0, st);
     if (int rc = dense_nn_launch(X, W, a->ax.p, a->n, feat, feat, stream)) return rc;  // P = X W, once per call
-    a->launches += 2;  // split_w_kernel + dense_tf32x3_ws_kernel
+    a->launches += dense_nn_launches(a->n, feat, feat);
     if (int rc = prof_agg_empty(a, st)) return rc;
     if (int rc = mlp_run_core(a, a->ax.p, Y, feat, scheduled, st)) return rc;
     PROF_RECORD(a, 3, st);

@@ -486,11 +486,20 @@ __global__ void __launch_bounds__(256) dense_simt_kernel(const float *__restrict
             if (row0 + ty * 4 + i < M && col0 + tx * 4 + j < N) C[(size_t)(row0 + ty * 4 + i) * N + col0 + tx * 4 + j] = acc[i][j];
 }
 
+// widths the tcgen05 kernel takes; every other product goes through dense_simt_kernel
+static bool dense_on_tensor_cores(int N, int K) { return N >= 32 && K >= 32 && N <= 256 && K <= 256 && N % 32 == 0 && K % 32 == 0; }
+
+int dense_nn_launches(int64_t M, int N, int K)
+{
+    if (M <= 0) return 0;
+    return dense_on_tensor_cores(N, K) ? 2 : (int)((M + (int64_t)65535 * 64 - 1) / ((int64_t)65535 * 64));
+}
+
 int dense_nn_launch(const float *A, const float *B, float *C, int64_t M, int N, int K, void *stream)
 {
     cudaStream_t st = (cudaStream_t)stream;
     if (N < 1 || K < 1) return set_error(GNNAGG_ERR_ARG, "dense combination: feat_in and feat_out must be positive");
-    if (N < 32 || K < 32 || N > 256 || K > 256 || (N % 32) || (K % 32)) {
+    if (!dense_on_tensor_cores(N, K)) {
         if (M <= 0) return GNNAGG_OK;
         const dim3 grid((unsigned)((N + 63) / 64), (unsigned)((M + 63) / 64));
         if (grid.y > 65535u * 16u) return set_error(GNNAGG_ERR_ARG, "dense combination: too many rows for the generic kernel");

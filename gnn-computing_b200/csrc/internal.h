@@ -55,6 +55,9 @@ int sample_subgraph_device(const int *d_ptr, const int *d_idx, const int *d_item
 
 // dense combination on tcgen05 (dense_tc.cu); stream is a cudaStream_t
 int dense_nn_launch(const float *A, const float *B, float *C, int64_t M, int N, int K, void *stream);
+// kernels dense_nn_launch issues for that product: split_w_kernel + the tcgen05 kernel, or the plain fp32 kernel once
+// per 65535 * 64 rows
+int dense_nn_launches(int64_t M, int N, int K);
 // loads the combination kernels and their per-device state ahead of the first launch (dense_tc.cu)
 void dense_preload();
 

@@ -504,6 +504,9 @@ class Aggregator:
 
     # --- per-edge MLP aggregator (aggr_nn.h)
     def mlp_run(self, X, W, Y, scheduled=False):
+        F = X.shape[1]
+        if tuple(W.shape) != (F, F):
+            raise GnnaggError("mlp_run: W must be [%d, %d] for X of width %d, got %s" % (F, F, F, tuple(W.shape)))
         check(lib().gnnagg_mlp_run(self.h, _f32(X, "X"), _f32(W, "W"), _f32(Y, "Y"), X.shape[1], int(scheduled), _stream()))
         return Y
 

@@ -215,8 +215,10 @@ int gnnagg_each_div(gnnagg_aggregator *a, const float *in_center, float *inout_v
 /* per-edge MLP aggregation  Y[v,:] = sum_{u in N(v)} ReLU((X[v,:] + X[u,:]) * W),  W row-major [feat, feat].
  * replaces Aggregator_MLP::run + aggr_mlp / aggr_mlp_target (include/aggr_nn.h:51-341; there feat = 32 only and
  * a 32x32 mat-vec per EDGE).  Here the projection is hoisted out of the edge loop: (x_v + x_u) W = P[v] + P[u]
- * with P = X W computed once on the tensor cores (gnnagg_dense_nn), so an edge costs one gathered row and
- * `feat` adds.  feat a multiple of 32 <= 256; scheduled = 1 uses the current schedule (RED combination). */
+ * with P = X W computed once (gnnagg_dense_nn), so an edge costs one gathered row and `feat` adds.  feat is a
+ * multiple of 4 in [4, 1024], checked before anything runs (GNNAGG_ERR_ARG otherwise); the projection runs on the
+ * tensor cores in 3xTF32 for multiples of 32 up to 256 and through the plain fp32 kernel for any other width.
+ * scheduled = 1 uses the current schedule (RED combination). */
 int gnnagg_mlp_run(gnnagg_aggregator *a, const float *X, const float *W, float *Y, int feat, int scheduled,
                    void *stream);
 
@@ -401,6 +403,7 @@ int64_t gnnagg_dist_launch_count(const gnnagg_dist *d);
 int gnnagg_gcn_run_host(gnnagg_aggregator *a, const float *h_X, float *h_Y, int feat, int scheduled, void *stream);
 int gnnagg_gcn_layer_host(gnnagg_aggregator *a, const float *h_X, const float *h_W, float *h_H, int feat_in,
                           int feat_out, int scheduled, void *stream);
+/* gnnagg_gat_run_host sizes h_X and h_att by num_v rows: square graph only (num_src = num_v), like the GCN calls */
 int gnnagg_gat_run_host(gnnagg_aggregator *a, const float *h_X, const float *h_att, float *h_Y, int feat,
                         float slope, int scheduled, void *stream);
 
