@@ -34,7 +34,7 @@ struct AggParams {
     const float *__restrict__ val;       // GCN edge values; unused for GAT
     const int *__restrict__ target;      // scheduled mode: output row of every group
     const int *__restrict__ item_row;    // row containing edge k*kFineItem
-    const void *__restrict__ X;          // [*, F] fp32, or bf16 bit patterns for the XBF16 instances of the GCN mode
+    const void *__restrict__ X;          // [*, F] fp32, or bf16 bit patterns for the XBF16 instances
     const float *__restrict__ att;       // GAT attention table [n,2]
     const float *__restrict__ P;         // MLP: projected features P = X*W, [n, F] (also the gather source); SDDMM: X2
     float *__restrict__ Y;               // [n, F]
@@ -99,13 +99,15 @@ __device__ __forceinline__ float4 ldg_x4(const char *x)
 
 // WE = edges staged per warp: 512 normally, 128 for small graphs (4x more warps, shorter walks)
 // (5 resident CTAs per SM for the small-graph variant -- 48 registers -- measured on the arxiv shape: no change.)
-// XBF16 (GCN only): X holds bf16.  The lane mapping, items and carries are those of the fp32 run of the same width;
-// each lane gathers 8 bytes where it gathered 16 and runs the same FMAs on the widened values, so the result equals the
-// fp32 run on the widened X bit for bit.
+// XBF16 (GCN, GAT, and pass 1 of the GAT backward): X holds bf16.  The lane mapping, items and carries are those of
+// the fp32 run of the same width; each lane gathers 8 bytes where it gathered 16 and runs the same FMAs / dot products
+// on the widened values, so the result equals the fp32 run on the widened X bit for bit.  The other operands (att, the
+// dY row of pass 1) stay fp32.
 template <int LPR, int NV, int MODE, bool SCHED, int WE, bool XBF16 = false>
 __global__ void __launch_bounds__(kCtaThreads, (WE < 512) ? 4 : 3) agg_kernel(const AggParams p)
 {
-    static_assert(!XBF16 || MODE == kModeGCN, "bf16 X is a GCN-only operand");
+    static_assert(!XBF16 || MODE == kModeGCN || MODE == kModeGAT || (MODE == kModeGATBWD && !SCHED),
+                  "bf16 X is an operand of the GCN and GAT aggregations and of pass 1 of the GAT backward");
     using XT = typename std::conditional<XBF16, uint16_t, float>::type;
     constexpr int kWarpEdges = WE;            // shadows the namespace-level default
     constexpr int VPW = 32 / LPR;             // virtual warps per warp

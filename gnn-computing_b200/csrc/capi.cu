@@ -375,10 +375,11 @@ static AggKernel agg_kernel_for(int WE, int F)
          : F <= 128 ? agg_kernel<32, 1, MODE, SCHED, kWarpEdges, XBF16>
                     : agg_kernel<32, 2, MODE, SCHED, kWarpEdges, XBF16>;
 }
+// (bf16 X: the GCN and GAT aggregations, and pass 1 of the GAT backward, which is never scheduled)
 template <int MODE, bool SCHED>
 static AggKernel agg_kernel_for(int WE, int F, bool xbf16)
 {
-    if constexpr (MODE == kModeGCN)
+    if constexpr (MODE == kModeGCN || MODE == kModeGAT || (MODE == kModeGATBWD && !SCHED))
         if (xbf16) return agg_kernel_for<MODE, SCHED, true>(WE, F);
     return agg_kernel_for<MODE, SCHED>(WE, F);
 }
@@ -423,7 +424,7 @@ static const LongRows *long_rows_of(View &v, const AggParams &p, int EB, cudaStr
     return &v.long_rows.back();
 }
 
-// xbf16: p.X holds bf16 (GCN only)
+// xbf16: p.X holds bf16 (GCN, GAT, pass 1 of the GAT backward)
 template <int MODE, bool SCHED>
 static int launch_agg(View &v, AggParams p, cudaStream_t st, bool xbf16 = false)
 {
@@ -466,8 +467,8 @@ static int launch_agg(View &v, AggParams p, cudaStream_t st, bool xbf16 = false)
 
 static int aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
-// the gathered operand of a GCN aggregation: fp32 X (16-byte aligned), or bf16 bit patterns (8-byte aligned) that the
-// kernel widens exactly to fp32
+// the gathered operand of a GCN or GAT aggregation (or of pass 1 of the GAT backward): fp32 X (16-byte aligned), or
+// bf16 bit patterns (8-byte aligned) that the kernel widens exactly to fp32
 struct GatherX {
     const void *p;
     bool bf16;
@@ -596,16 +597,16 @@ static void row_chunks(const int *hp, int n, int m, int chunks, int *bounds)
     bounds[chunks] = n;
 }
 
-static int gat_run_core(gnnagg_aggregator *a, const float *X, const float *att, float *Y, int F, float slope,
+static int gat_run_core(gnnagg_aggregator *a, GatherX X, const float *att, float *Y, int F, float slope,
                         int scheduled, cudaStream_t st)
 {
     if (a && a->n == 0) return GNNAGG_OK;
-    if (!a || !X || !Y || !att) return set_error(GNNAGG_ERR_ARG, "gnnagg_gat_run: NULL argument");
+    if (!a || !X.p || !Y || !att) return set_error(GNNAGG_ERR_ARG, "gnnagg_gat_run: NULL argument");
     if (int rc = check_feat(F)) return rc;
-    if (!aligned16(X) || !aligned16(Y)) return set_error(GNNAGG_ERR_ARG, "X and Y must be 16-byte aligned");
+    if (int rc = check_xy(X, Y)) return rc;
     if (int rc = a->den_row.ensure((size_t)a->n)) return rc;
     AggParams p{};
-    p.X = X;
+    p.X = X.p;
     p.Y = Y;
     p.att = att;
     p.F = F;
@@ -618,7 +619,7 @@ static int gat_run_core(gnnagg_aggregator *a, const float *X, const float *att, 
         if (int rc = a->newval.ensure((size_t)a->sched.edges)) return rc;
         p.newval = a->newval.p;
         p.bulk_ok = aligned16(p.idx);
-        if (int rc = launch_agg<kModeGAT, true>(*a, p, st)) return rc;
+        if (int rc = launch_agg<kModeGAT, true>(*a, p, st, X.bf16)) return rc;
         const int64_t total4 = (int64_t)a->n * F / 4;
         gat_scale_kernel<<<(unsigned)cdiv(total4, 256), 256, 0, st>>>(Y, a->den_row.p, F, total4);
         LAUNCH_CHECK(a);
@@ -635,7 +636,7 @@ static int gat_run_core(gnnagg_aggregator *a, const float *X, const float *att, 
     p.carry = a->carry.p;
     p.carry_den = a->carry_den.p;
     p.bulk_ok = aligned16(p.idx);
-    return launch_agg<kModeGAT, false>(*a, p, st);
+    return launch_agg<kModeGAT, false>(*a, p, st, X.bf16);
 }
 
 static int mlp_run_core(gnnagg_aggregator *a, const float *P, float *Y, int F, int scheduled, cudaStream_t st)
@@ -783,7 +784,7 @@ static int gcn_run_impl(gnnagg_aggregator *a, GatherX X, float *Y, int F, int sc
     return GNNAGG_OK;
 }
 
-static int gat_run_impl(gnnagg_aggregator *a, const float *X, const float *att, float *Y, int F, float slope,
+static int gat_run_impl(gnnagg_aggregator *a, GatherX X, const float *att, float *Y, int F, float slope,
                         int scheduled, cudaStream_t st)
 {
     if (a) {
@@ -917,6 +918,95 @@ static int gcn_backward_impl(gnnagg_aggregator *a, GatherX dY, float *dX, int fe
         t.val_gen = a->val_gen;
     }
     return gcn_run_core(t.v, dY, dX, feat, 0, st);
+}
+
+// X (fp32 or bf16) is read by pass 1 only; Y, dY and the other operands are fp32 for both element types of X
+static int gat_backward_impl(gnnagg_aggregator *a, GatherX X, const float *att, const float *w, const float *den,
+                             const float *Y, const float *dY, float *dX, float *datt, int feat, float slope, cudaStream_t st)
+{
+    if (!a || !X.p || !Y || !dY || !dX || !datt || (!att && !w))
+        return set_error(GNNAGG_ERR_ARG, "gnnagg_gat_backward: NULL argument (att or w must be given)");
+    if (!a->tr) return set_error(GNNAGG_ERR_STATE, "gnnagg_gat_backward: gnnagg_transpose_build has not run");
+    if (int rc = check_feat(feat)) return rc;
+    if (X.bf16) {
+        if ((reinterpret_cast<uintptr_t>(X.p) & 7) || !aligned16(Y) || !aligned16(dY) || !aligned16(dX))
+            return set_error(GNNAGG_ERR_ARG, "X (bf16) must be 8-byte aligned, Y, dY and dX 16-byte aligned");
+    } else if (!aligned16(X.p) || !aligned16(Y) || !aligned16(dY) || !aligned16(dX)) {
+        return set_error(GNNAGG_ERR_ARG, "X, Y, dY and dX must be 16-byte aligned");
+    }
+    Transpose &tr = *a->tr;
+    View &t = tr.v;
+    // every row < n gets its destination half and every row < num_src its source half from the kernels below; only a
+    // rectangular block leaves entries of the [max(n, num_src), 2] table that nobody writes
+    const int rows = a->n > t.n ? a->n : t.n;
+    if (a->n != t.n || a->m == 0) CUDA_TRY(cudaMemsetAsync(datt, 0, (size_t)rows * 2 * sizeof(float), st));
+    if (a->m == 0) {
+        CUDA_TRY(cudaMemsetAsync(dX, 0, (size_t)t.n * feat * sizeof(float), st));
+        return GNNAGG_OK;
+    }
+    const int EB = item_edges_for(*a, feat, a->m);
+    const int EBt = item_edges_for(t, feat, a->m);
+    if (int rc = a->bwd_c.ensure((size_t)a->n)) return rc;
+    if (int rc = a->bwd_wt.ensure((size_t)a->m)) return rc;
+    if (int rc = a->bwd_part.ensure((size_t)a->n)) return rc;
+    if (int rc = a->bwd_carry.ensure((size_t)cdiv(a->m, EB) + 1)) return rc;
+    if (int rc = t.carry.ensure((size_t)cdiv(a->m, EBt) * feat)) return rc;
+    if (int rc = t.carry_den.ensure((size_t)cdiv(a->m, EBt))) return rc;
+    if (int rc = t.den_row.ensure((size_t)t.n)) return rc;
+    const bool large = a->m >= kSmallGraphEdges;  // (w, t) of the graph does not stay in L2: see step 4
+    if (large)
+        if (int rc = a->bwd_t.ensure((size_t)a->m)) return rc;
+    // 1. per destination row: c_v = <Y[v], dY[v]>
+    gat_bwd_rowinfo_kernel<<<(unsigned)cdiv((int64_t)a->n * 8, 256), 256, 0, st>>>(Y, dY, a->bwd_c.p, a->n, feat);
+    LAUNCH_CHECK(a);
+    // 2. pass 1 over the CSR: g_e = <X[u], dY[v]> (the SDDMM traversal), per edge (w_e, t_e), per row their sums
+    {
+        AggParams p{};
+        p.X = X.p;
+        p.P = dY;
+        p.att = att;
+        p.val = w;
+        p.bwd_c = a->bwd_c.p;
+        p.bwd_wt = a->bwd_wt.p;
+        p.bwd_part = a->bwd_part.p;
+        p.bwd_carry = a->bwd_carry.p;
+        p.F = feat;
+        p.slope = slope;
+        set_view(p, *a);
+        p.bulk_ok = aligned16(p.idx) && (att || aligned16(w));
+        if (int rc = launch_agg<kModeGATBWD, false>(*a, p, st, X.bf16)) return rc;
+    }
+    // 3. rows closed: 1 / D_v and the destination half of the attention gradient
+    launch_dep(gat_bwd_rowfinal_kernel, (unsigned)cdiv((int64_t)a->n * 8, 256), 256, st, a->d_ptr, a->bwd_part.p,
+               a->bwd_carry.p, den, a->bwd_c.p, datt, a->n, EB);
+    LAUNCH_CHECK(a);
+    if (large) {
+        // 4a. large graphs: (w, t) permuted into transposed order by a streaming kernel, then the source half as a row sum
+        //     and dX as the plain aggregation over the transposed CSR with edge values alpha
+        launch_dep(gat_bwd_permute_kernel, (unsigned)cdiv(a->m, 256), 256, st, (const float2 *)a->bwd_wt.p,
+                   (const int *)tr.perm.p, (const int *)tr.idx.p, (const float2 *)a->bwd_c.p, tr.val.p, a->bwd_t.p, a->m);
+        LAUNCH_CHECK(a);
+        tr.val_gen = 0;  // tr.val no longer mirrors the GCN edge values
+        if (int rc = rowsum_impl(t, a->bwd_t.p, datt + 1, st, 2)) return rc;
+        return gcn_run_core(t, dY, dX, feat, 0, st);
+    }
+    // 4b. pass 2 over the transposed CSR: dX[u] = sum_e alpha_e dY[v] and the source half sum_e ds_e, weights formed on
+    //     the fly from (w, t) through tr.perm and 1 / D_v ((w, t) of a small graph stays in L2)
+    AggParams p{};
+    p.X = dY;
+    p.Y = dX;
+    p.val = reinterpret_cast<const float *>(tr.perm.p);
+    p.bwd_c = a->bwd_c.p;
+    p.bwd_wt = a->bwd_wt.p;
+    p.rsum = datt + 1;
+    p.rsum_stride = 2;
+    p.F = feat;
+    set_view(p, t);
+    p.carry = t.carry.p;
+    p.carry_den = t.carry_den.p;
+    p.den_row = t.den_row.p;
+    p.bulk_ok = aligned16(p.idx) && aligned16(p.val);
+    return launch_agg<kModeGATBWD2, false>(t, p, st);
 }
 
 }  // namespace gnnagg
@@ -1211,6 +1301,12 @@ int gnnagg_gat_run(gnnagg_aggregator *a, const float *X, const float *att, float
     return gat_run_impl(a, X, att, Y, feat, slope, scheduled, (cudaStream_t)stream);
 }
 
+int gnnagg_gat_run_bf16(gnnagg_aggregator *a, const uint16_t *X, const float *att, float *Y, int feat, float slope,
+                        int scheduled, void *stream)
+{
+    return gat_run_impl(a, X, att, Y, feat, slope, scheduled, (cudaStream_t)stream);
+}
+
 int gnnagg_dense_nn(const float *A, const float *B, float *C, int64_t M, int N, int K, void *stream)
 {
     if (!A || !B || !C || M < 0) return set_error(GNNAGG_ERR_ARG, "gnnagg_dense_nn: bad argument");
@@ -1397,86 +1493,13 @@ int gnnagg_gcn_backward_bf16(gnnagg_aggregator *a, const uint16_t *dY, float *dX
 int gnnagg_gat_backward(gnnagg_aggregator *a, const float *X, const float *att, const float *w, const float *den,
                         const float *Y, const float *dY, float *dX, float *datt, int feat, float slope, void *stream)
 {
-    if (!a || !X || !Y || !dY || !dX || !datt || (!att && !w))
-        return set_error(GNNAGG_ERR_ARG, "gnnagg_gat_backward: NULL argument (att or w must be given)");
-    if (!a->tr) return set_error(GNNAGG_ERR_STATE, "gnnagg_gat_backward: gnnagg_transpose_build has not run");
-    if (int rc = check_feat(feat)) return rc;
-    if (!aligned16(X) || !aligned16(Y) || !aligned16(dY) || !aligned16(dX))
-        return set_error(GNNAGG_ERR_ARG, "X, Y, dY and dX must be 16-byte aligned");
-    cudaStream_t st = (cudaStream_t)stream;
-    Transpose &tr = *a->tr;
-    View &t = tr.v;
-    // every row < n gets its destination half and every row < num_src its source half from the kernels below; only a
-    // rectangular block leaves entries of the [max(n, num_src), 2] table that nobody writes
-    const int rows = a->n > t.n ? a->n : t.n;
-    if (a->n != t.n || a->m == 0) CUDA_TRY(cudaMemsetAsync(datt, 0, (size_t)rows * 2 * sizeof(float), st));
-    if (a->m == 0) {
-        CUDA_TRY(cudaMemsetAsync(dX, 0, (size_t)t.n * feat * sizeof(float), st));
-        return GNNAGG_OK;
-    }
-    const int EB = item_edges_for(*a, feat, a->m);
-    const int EBt = item_edges_for(t, feat, a->m);
-    if (int rc = a->bwd_c.ensure((size_t)a->n)) return rc;
-    if (int rc = a->bwd_wt.ensure((size_t)a->m)) return rc;
-    if (int rc = a->bwd_part.ensure((size_t)a->n)) return rc;
-    if (int rc = a->bwd_carry.ensure((size_t)cdiv(a->m, EB) + 1)) return rc;
-    if (int rc = t.carry.ensure((size_t)cdiv(a->m, EBt) * feat)) return rc;
-    if (int rc = t.carry_den.ensure((size_t)cdiv(a->m, EBt))) return rc;
-    if (int rc = t.den_row.ensure((size_t)t.n)) return rc;
-    const bool large = a->m >= kSmallGraphEdges;  // (w, t) of the graph does not stay in L2: see step 4
-    if (large)
-        if (int rc = a->bwd_t.ensure((size_t)a->m)) return rc;
-    // 1. per destination row: c_v = <Y[v], dY[v]>
-    gat_bwd_rowinfo_kernel<<<(unsigned)cdiv((int64_t)a->n * 8, 256), 256, 0, st>>>(Y, dY, a->bwd_c.p, a->n, feat);
-    LAUNCH_CHECK(a);
-    // 2. pass 1 over the CSR: g_e = <X[u], dY[v]> (the SDDMM traversal), per edge (w_e, t_e), per row their sums
-    {
-        AggParams p{};
-        p.X = X;
-        p.P = dY;
-        p.att = att;
-        p.val = w;
-        p.bwd_c = a->bwd_c.p;
-        p.bwd_wt = a->bwd_wt.p;
-        p.bwd_part = a->bwd_part.p;
-        p.bwd_carry = a->bwd_carry.p;
-        p.F = feat;
-        p.slope = slope;
-        set_view(p, *a);
-        p.bulk_ok = aligned16(p.idx) && (att || aligned16(w));
-        if (int rc = launch_agg<kModeGATBWD, false>(*a, p, st)) return rc;
-    }
-    // 3. rows closed: 1 / D_v and the destination half of the attention gradient
-    launch_dep(gat_bwd_rowfinal_kernel, (unsigned)cdiv((int64_t)a->n * 8, 256), 256, st, a->d_ptr, a->bwd_part.p,
-               a->bwd_carry.p, den, a->bwd_c.p, datt, a->n, EB);
-    LAUNCH_CHECK(a);
-    if (large) {
-        // 4a. large graphs: (w, t) permuted into transposed order by a streaming kernel, then the source half as a row sum
-        //     and dX as the plain aggregation over the transposed CSR with edge values alpha
-        launch_dep(gat_bwd_permute_kernel, (unsigned)cdiv(a->m, 256), 256, st, (const float2 *)a->bwd_wt.p,
-                   (const int *)tr.perm.p, (const int *)tr.idx.p, (const float2 *)a->bwd_c.p, tr.val.p, a->bwd_t.p, a->m);
-        LAUNCH_CHECK(a);
-        tr.val_gen = 0;  // tr.val no longer mirrors the GCN edge values
-        if (int rc = rowsum_impl(t, a->bwd_t.p, datt + 1, st, 2)) return rc;
-        return gcn_run_core(t, dY, dX, feat, 0, st);
-    }
-    // 4b. pass 2 over the transposed CSR: dX[u] = sum_e alpha_e dY[v] and the source half sum_e ds_e, weights formed on
-    //     the fly from (w, t) through tr.perm and 1 / D_v ((w, t) of a small graph stays in L2)
-    AggParams p{};
-    p.X = dY;
-    p.Y = dX;
-    p.val = reinterpret_cast<const float *>(tr.perm.p);
-    p.bwd_c = a->bwd_c.p;
-    p.bwd_wt = a->bwd_wt.p;
-    p.rsum = datt + 1;
-    p.rsum_stride = 2;
-    p.F = feat;
-    set_view(p, t);
-    p.carry = t.carry.p;
-    p.carry_den = t.carry_den.p;
-    p.den_row = t.den_row.p;
-    p.bulk_ok = aligned16(p.idx) && aligned16(p.val);
-    return launch_agg<kModeGATBWD2, false>(t, p, st);
+    return gat_backward_impl(a, X, att, w, den, Y, dY, dX, datt, feat, slope, (cudaStream_t)stream);
+}
+
+int gnnagg_gat_backward_bf16(gnnagg_aggregator *a, const uint16_t *X, const float *att, const float *w, const float *den,
+                             const float *Y, const float *dY, float *dX, float *datt, int feat, float slope, void *stream)
+{
+    return gat_backward_impl(a, X, att, w, den, Y, dY, dX, datt, feat, slope, (cudaStream_t)stream);
 }
 
 int gnnagg_sample_subgraph(gnnagg_aggregator *a, int *d_active, int fanout, int layer_num, uint64_t seed, int **d_vertexset,

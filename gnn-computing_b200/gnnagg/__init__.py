@@ -80,6 +80,7 @@ _SIGS = {
     "gnnagg_gcn_layer_bf16": (C.c_int, [C.c_void_p] * 5 + [C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "gnnagg_dense_nn": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p]),
     "gnnagg_gat_run": (C.c_int, [C.c_void_p] * 4 + [C.c_int, C.c_float, C.c_int, C.c_void_p]),
+    "gnnagg_gat_run_bf16": (C.c_int, [C.c_void_p] * 4 + [C.c_int, C.c_float, C.c_int, C.c_void_p]),
     "gnnagg_gat_edge_weights": (C.c_void_p, [C.c_void_p]),
     "gnnagg_edge_softmax": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, C.c_void_p]),
     "gnnagg_u_add_v": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
@@ -92,6 +93,7 @@ _SIGS = {
     "gnnagg_gcn_backward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "gnnagg_gcn_backward_bf16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "gnnagg_gat_backward": (C.c_int, [C.c_void_p] * 9 + [C.c_int, C.c_float, C.c_void_p]),
+    "gnnagg_gat_backward_bf16": (C.c_int, [C.c_void_p] * 9 + [C.c_int, C.c_float, C.c_void_p]),
     "gnnagg_sample_subgraph": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_uint64] + [C.POINTER(C.c_void_p)] * 3 +
                                [C.POINTER(C.c_int)] * 2 + [C.c_void_p]),
     "gnnagg_device_free": (C.c_int, [C.c_void_p]),
@@ -285,7 +287,7 @@ def _f32(t, name, cuda=True):
 
 
 def _bf16(t, name, cuda=True):
-    """bfloat16 torch operand (the gathered X / dY of the bf16 GCN entry points, or the host X shard of
+    """bfloat16 torch operand (the gathered X / dY of the bf16 GCN and GAT entry points, or the host X shard of
     gnnagg_dist_gcn_layer_host_bf16 with cuda=False); numpy has no bf16, so numpy arrays are not accepted"""
     import torch
 
@@ -478,9 +480,15 @@ class Aggregator:
                                          _stream()))
         return H
 
-    # --- GAT
+    # --- GAT (gat_run / gat_backward take a float32 X only; the _bf16 forms take a bfloat16 X, every other operand of
+    # both is float32)
     def gat_run(self, X, att, Y, slope=0.2, scheduled=False):
         check(lib().gnnagg_gat_run(self.h, _f32(X, "X"), _f32(att, "att"), _f32(Y, "Y"), X.shape[1], slope, int(scheduled), _stream()))
+        return Y
+
+    def gat_run_bf16(self, X, att, Y, slope=0.2, scheduled=False):
+        check(lib().gnnagg_gat_run_bf16(self.h, _bf16(X, "X"), _f32(att, "att"), _f32(Y, "Y"), X.shape[1], slope,
+                                        int(scheduled), _stream()))
         return Y
 
     def gat_edge_weights_ptr(self):
@@ -544,6 +552,12 @@ class Aggregator:
     def gat_backward(self, X, att, Y, dY, dX, datt, slope=0.2, w=None, den=None):
         check(lib().gnnagg_gat_backward(self.h, _f32(X, "X"), _f32(att, "att"), _f32(w, "w"), _f32(den, "den"), _f32(Y, "Y"), _f32(dY, "dY"), _f32(dX, "dX"), _f32(datt, "datt"),
                                         X.shape[1], slope, _stream()))
+        return dX, datt
+
+    def gat_backward_bf16(self, X, att, Y, dY, dX, datt, slope=0.2, w=None, den=None):
+        check(lib().gnnagg_gat_backward_bf16(self.h, _bf16(X, "X"), _f32(att, "att"), _f32(w, "w"), _f32(den, "den"),
+                                             _f32(Y, "Y"), _f32(dY, "dY"), _f32(dX, "dX"), _f32(datt, "datt"), X.shape[1],
+                                             slope, _stream()))
         return dX, datt
 
     # --- sub-graph samplers (sample.h)

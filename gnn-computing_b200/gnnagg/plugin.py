@@ -140,27 +140,33 @@ class GCNAggregate(torch.autograd.Function):
 
 class GATAggregate(torch.autograd.Function):
     """Y = fused GAT aggregation of X with the attention table att [n, 2] (destination term, source term), slope 0.2
-    as in the reference (aggr_gat.h:339).  backward: full gradient w.r.t. X and att."""
+    as in the reference (aggr_gat.h:339).  backward: full gradient w.r.t. X and att.  X may be float32 or bfloat16: a
+    bf16 X is gathered as stored (gnnagg_gat_run_bf16 / gnnagg_gat_backward_bf16) and kept for the backward at half
+    the memory.  att may be float32 or bfloat16; it is widened to float32 once per forward.  Y is float32.  dX and
+    datt are computed in float32 and rounded once to the dtypes of X and att."""
 
     @staticmethod
     def forward(ctx, at, X, att, slope=0.2):
         agg = _get(at)
         X, att = X.contiguous(), att.contiguous()
         _check(X, att)
+        att32 = att.float() if att.dtype == torch.bfloat16 else att
         Y = torch.empty((agg.n, X.shape[1]), device=X.device, dtype=torch.float32)
-        agg.gat_run(X, att, Y, slope, False)
-        ctx.at, ctx.slope = at, slope
-        ctx.save_for_backward(X, att, Y)
+        run = agg.gat_run_bf16 if X.dtype == torch.bfloat16 else agg.gat_run
+        run(X, att32, Y, slope, False)
+        ctx.at, ctx.slope, ctx.att_dtype = at, slope, att.dtype
+        ctx.save_for_backward(X, att32, Y)
         return Y
 
     @staticmethod
     def backward(ctx, dY):
         X, att, Y = ctx.saved_tensors
         agg = _transposed(_get(ctx.at), X.shape[0])
-        dX = torch.empty_like(X)
+        dX = torch.empty(X.shape, device=X.device, dtype=torch.float32)
         datt = torch.empty((max(agg.n, X.shape[0]), 2), device=X.device, dtype=torch.float32)
-        agg.gat_backward(X, att, Y, dY.contiguous(), dX, datt, ctx.slope)
-        return None, dX, datt[: att.shape[0]], None
+        backward = agg.gat_backward_bf16 if X.dtype == torch.bfloat16 else agg.gat_backward
+        backward(X, att, Y, dY.contiguous(), dX, datt, ctx.slope)
+        return None, dX.to(X.dtype), datt[: att.shape[0]].to(ctx.att_dtype), None
 
 
 def gcn_aggregate(at, X, scheduled=False):

@@ -275,6 +275,23 @@ int gnnagg_gcn_run_acc_bf16(gnnagg_aggregator *a, const uint16_t *X, float *Y, i
 int gnnagg_gcn_run_rows_bf16(gnnagg_aggregator *a, const uint16_t *X, float *Y, int feat, int accumulate, int row_lo,
                              int row_hi, void *stream);
 
+/* ---- GAT aggregation from bf16 features ------------------------------------------------------------------
+ * gnnagg_gat_run and gnnagg_gat_backward with X stored in bf16: X is bf16 bit patterns, 8-byte aligned, [rows, feat]
+ * row-major.  att, w, den, Y, dY, dX and datt stay fp32 (Y, dY and dX 16-byte aligned); feat is a multiple of 4 in
+ * [4, 1024]; att or w must be given, den is optional; every argument error is reported before anything is launched.
+ * Each bf16 value is widened exactly to fp32 on load and then used as in the fp32 run, with the same items, carries
+ * and fix-up order, so:
+ *   - the un-scheduled forward, and the backward on both of its routes (small graphs: pass 2 over the transposed CSR;
+ *     large graphs: permute, row sum and the plain aggregation), equal the fp32 entry point on the widened X bit for bit;
+ *   - the scheduled forward matches it up to the arbitrary RED.ADD order; the un-normalised weights it leaves in
+ *     gnnagg_gat_edge_weights() equal the fp32 run's bit for bit, because they do not depend on X.
+ * In the backward only the traversal that gathers X (pass 1, <X[u], dY[v]>) reads bf16; dY is gathered in fp32.
+ * Routing, profiling (gnnagg_profile_read) and the launch count are those of the fp32 entry point. */
+int gnnagg_gat_run_bf16(gnnagg_aggregator *a, const uint16_t *X, const float *att, float *Y, int feat, float slope,
+                        int scheduled, void *stream);
+int gnnagg_gat_backward_bf16(gnnagg_aggregator *a, const uint16_t *X, const float *att, const float *w, const float *den,
+                             const float *Y, const float *dY, float *dX, float *datt, int feat, float slope, void *stream);
+
 /* ---- sub-graph samplers (SURVEY §8(f) rank 4) -------------------------------------------------------------
  * replaces sampleVertex (include/sample.h:131-200) and sampleVertexSampleNeighbor (:274-357).
  * d_active [num_v]: non-zero marks the seed vertices; on return it holds the 0/1 set after layer_num - 1 hops
@@ -454,7 +471,7 @@ int gnnagg_merged_dev(const gnnagg_aggregator *a, const int **ptr, const int **i
  * or force 128 / 512.  Results do not depend on it beyond fp32 summation order. */
 int gnnagg_set_warp_edges(gnnagg_aggregator *a, int warp_edges);
 
-/* per-kernel device timing of the LAST gnnagg_gcn_run / gnnagg_gat_run / gnnagg_gcn_layer call:
+/* per-kernel device timing of the LAST gnnagg_gcn_run / gnnagg_gat_run / gnnagg_gcn_layer call (or its _bf16 form):
  * when enabled the library brackets its launches with CUDA events on the caller's stream.
  * gnnagg_profile_read synchronises on those events and returns milliseconds in
  * ms[0] = aggregation kernel, ms[1] = split-row fix-up (or memset+scale in scheduled mode),
