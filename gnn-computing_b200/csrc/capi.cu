@@ -688,7 +688,6 @@ static int ensure_slices(gnnagg_aggregator *a, std::unique_ptr<Slices> &set, int
             v.d_val = s->val.p + s->off[c];
             v.n = a->n;
             v.m = s->cnt[c];
-            v.warp_edges = a->warp_edges ? a->warp_edges : (a->m < kSmallGraphEdges ? 128 : kWarpEdges);  // as the whole graph
             if (compact && c > 0) {
                 // slices behind the first only ADD to rows that have edges in them: keep those rows only (slice 0 stays
                 // complete: it is the pass that writes every row, zeros included)
@@ -715,6 +714,10 @@ static int ensure_slices(gnnagg_aggregator *a, std::unique_ptr<Slices> &set, int
         }
         set->val_gen = a->val_gen;
     }
+    // the item size follows the root's setting on every run, as in the merged and transposed views (carries and long-row
+    // records are kept per item size); automatic decides on the whole graph's edge count, not on a slice's
+    const int we = a->warp_edges ? a->warp_edges : (a->m < kSmallGraphEdges ? 128 : kWarpEdges);
+    for (Slices::Slice &sl : set->slice) sl.v.warp_edges = we;
     return GNNAGG_OK;
 }
 

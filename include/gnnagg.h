@@ -468,7 +468,8 @@ int gnnagg_merged_dev(const gnnagg_aggregator *a, const int **ptr, const int **i
 
 /* tuning knob (the reference's analogue is the BLOCK_SIZE argument of run(), aggr_gcn.h:381-386):
  * edges staged per warp by the aggregation kernels: 0 = automatic (128 below 4M edges, else 512),
- * or force 128 / 512.  Results do not depend on it beyond fp32 summation order. */
+ * or force 128 / 512.  Results do not depend on it beyond fp32 summation order.  It applies from the next run on,
+ * also to the views built earlier (transposed CSR, merged view, locality and host-pipeline source slices). */
 int gnnagg_set_warp_edges(gnnagg_aggregator *a, int warp_edges);
 
 /* per-kernel device timing of the LAST gnnagg_gcn_run / gnnagg_gat_run / gnnagg_gcn_layer call (or its _bf16 form):
