@@ -51,6 +51,9 @@ struct HaloFlags {
     uint32_t consumed[kMaxWorld];  // consumed[q]: last epoch receiver q finished reading what I pushed to it (written by q)
     uint32_t push_cnt[kMaxWorld];  // local: CTAs of the running push kernel towards q that are done
     uint32_t err;                  // first protocol error seen by a kernel of this rank (0 = none)
+    // backward (gnnagg_dist_gcn_backward), behind `err` so that the forward's offsets stay where they were
+    uint32_t grad_ready[kMaxWorld];  // grad_ready[q]: last backward epoch whose partial sums sender q has written into ITS G (written by q)
+    uint32_t grad_read[kMaxWorld];   // grad_read[p]: last backward epoch owner p finished reading MY G (written by p)
 };
 static_assert(sizeof(HaloFlags) <= kFlagBytes, "flags page too small");
 
@@ -124,6 +127,62 @@ __global__ void __launch_bounds__(32) halo_consumed_kernel(PeerTable peers, int 
 {
     const int p = threadIdx.x;
     if (p < world && p != rank) st_release_sys(&peers.flags[p]->consumed[rank], epoch);
+}
+
+// ---- backward: dX = A^T dY across ranks.  Every rank writes the partial sums of the remote sources it references into
+// its own G (peer-visible, laid out like an X buffer); every owner PULLS the rows meant for it and adds them to its dX.
+
+// waits until flags[p] has reached `epoch` for every p in `mask`; a timeout records code + p in *err
+__global__ void __launch_bounds__(32) grad_wait_kernel(const uint32_t *flags, uint32_t mask, uint32_t epoch, uint32_t *err,
+                                                       uint32_t code)
+{
+    const int p = threadIdx.x;
+    if (p < kMaxWorld && ((mask >> p) & 1u)) spin_until(flags + p, epoch, err, code + (uint32_t)p);
+}
+
+// raises this rank's entry of grad_ready (which = 0: "my G holds epoch e") or grad_read (which = 1: "I have read your G of
+// epoch e") at every peer; the fence orders the stream's earlier writes (G) before the flag at system scope
+__global__ void __launch_bounds__(32) grad_signal_kernel(PeerTable peers, int rank, int world, int which, uint32_t epoch)
+{
+    const int p = threadIdx.x;
+    __threadfence_system();
+    if (p < world && p != rank) st_release_sys(which ? &peers.flags[p]->grad_read[rank] : &peers.flags[p]->grad_ready[rank], epoch);
+}
+
+struct GradPeers {
+    const float4 *g[kMaxWorld];  // G of every peer (this rank's slot: unused)
+};
+
+// dX[rows[k], :] += G_q[r, :] for the return entries (q, r) of own row rows[k], in table order (peers ascending): each row
+// with remote contributions gets exactly one read-modify-write per step, no atomics, a fixed order of sums.  One thread per
+// 16-byte column chunk: the threads of a row read contiguous bytes of each peer row (remote loads over NVLink).
+__global__ void __launch_bounds__(256) grad_return_kernel(GradPeers peers, const int *__restrict__ rows, const int *__restrict__ off,
+                                                          const unsigned long long *__restrict__ ent, float4 *__restrict__ dX,
+                                                          int count, int F4)
+{
+    const int64_t t = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (t >= (int64_t)count * F4) return;
+    const int k = (int)(t / F4), c = (int)(t - (int64_t)k * F4);
+    const int lo = __ldg(off + k), hi = __ldg(off + k + 1);
+    float4 *out = dX + (int64_t)__ldg(rows + k) * F4 + c;
+    float4 acc = *out;
+#pragma unroll 4
+    for (int e = lo; e < hi; ++e) {
+        const unsigned long long en = __ldg(ent + e);  // peer in the high word, row of its G in the low word
+        const float4 v = peers.g[(int)(en >> 32)][(int64_t)(uint32_t)en * F4 + c];
+        acc.x += v.x, acc.y += v.y, acc.z += v.z, acc.w += v.w;
+    }
+    *out = acc;
+}
+
+// return entries of the rows peer `peer` wants from this owner in one round: key = own row, value = (peer, row of its G)
+__global__ void __launch_bounds__(256) grad_return_fill_kernel(const int *__restrict__ list, int count, int peer, int g_first,
+                                                               int *__restrict__ keys, unsigned long long *__restrict__ vals)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= count) return;
+    keys[i] = __ldg(list + i);
+    vals[i] = ((unsigned long long)(uint32_t)peer << 32) | (uint32_t)(g_first + i);
 }
 
 // dst[i, :] = X[rows[i], :] for the `count` rows receiver q wants from this owner (in this round): X is the own shard
@@ -465,6 +524,8 @@ struct DistBlob {
     uint64_t off_x[2], off_req, off_meta;
     int rounds;  // 1, or the row chunks of the row-pipelined mode: rows of recv_tab (in the buffer, at off_meta) in use
     cudaIpcMemHandle_t mem;
+    int backward;   // 1: gnnagg_dist_enable_backward ran; the G buffer sits at off_g
+    uint64_t off_g;
 };
 static_assert(sizeof(DistBlob) <= GNNAGG_DIST_BLOB_BYTES, "blob too large");
 
@@ -524,6 +585,19 @@ struct gnnagg_dist {
     int push_tma = 0;           // 1: rows staged through shared memory by bulk copies (halo_push_tma_kernel); 0: register version
     int same_device_ranks = 1;  // ranks (including this one) living on this rank's device: > 1 only in single-GPU tests
     int64_t launches = 0;
+    // backward (gnnagg_dist_enable_backward): the re-indexed block transposed on the GPU -- rows = own shard rows, then
+    // receive slots -- as an ordinary aggregator; G = [rows | num_recv] x feat fp32 inside the peer-visible allocation, at
+    // off_g; the return tables (built at connect): own rows that peers reference, ret_off[ret_rows + 1] into ret_ent
+    bool bwd_enabled = false;
+    int *bw_ptr = nullptr, *bw_idx = nullptr;
+    float *bw_val = nullptr;
+    gnnagg_aggregator *bwd = nullptr;
+    size_t off_g = 0;
+    size_t peer_off_g[kMaxWorld] = {0};
+    int *ret_row = nullptr, *ret_off = nullptr;
+    unsigned long long *ret_ent = nullptr;
+    int ret_rows = 0;
+    uint32_t bepoch = 0;
 };
 
 static HaloFlags *flags_of(char *base) { return reinterpret_cast<HaloFlags *>(base); }
@@ -538,6 +612,10 @@ static void close_peers(gnnagg_dist *d)
         d->send_rows[p] = nullptr;
         for (int c = 0; c < kMaxRounds; ++c) d->send_cnt[p][c] = 0;
     }
+    cudaFree(d->ret_row), cudaFree(d->ret_off), cudaFree(d->ret_ent);
+    d->ret_row = d->ret_off = nullptr;
+    d->ret_ent = nullptr;
+    d->ret_rows = 0;
     d->connected = d->world == 1 && d->base != nullptr;
 }
 
@@ -549,6 +627,11 @@ static void free_graph(gnnagg_dist *d)
         d->stage[s] = nullptr;
     }
     cudaFree(d->sl_ptr), cudaFree(d->sl_idx), cudaFree(d->sl_perm), cudaFree(d->sl_val);
+    if (d->bwd) gnnagg_destroy(d->bwd);
+    d->bwd = nullptr;
+    cudaFree(d->bw_ptr), cudaFree(d->bw_idx), cudaFree(d->bw_val);
+    d->bw_ptr = d->bw_idx = nullptr;
+    d->bw_val = nullptr;
     cudaFree(d->base);
     d->sl_ptr = d->sl_idx = d->sl_perm = nullptr;
     d->sl_val = nullptr;
@@ -559,6 +642,68 @@ static void free_graph(gnnagg_dist *d)
     d->prepared_feat = 0;
     d->connected = false;
     d->peer_base[d->rank] = nullptr;
+}
+
+// the return tables of the backward, built on the device from what connect copied (send_rows, peer_slot): for every own
+// row that peers reference, its entries (q, row of q's G) in ascending q.  The entries are appended peer by peer, stably
+// sorted by own row and run-length encoded into rows and offsets.
+static int build_return_tables(gnnagg_dist *d)
+{
+    struct Scratch {
+        int *keys = nullptr, *keys_sorted = nullptr, *counts = nullptr, *num_runs = nullptr;
+        unsigned long long *vals = nullptr;
+        void *tmp = nullptr;
+        ~Scratch() { cudaFree(keys), cudaFree(keys_sorted), cudaFree(counts), cudaFree(num_runs), cudaFree(vals), cudaFree(tmp); }
+    } s;
+    int64_t total = 0;
+    for (int q = 0; q < d->world; ++q)
+        for (int c = 0; c < d->rounds; ++c) total += d->send_cnt[q][c];
+    if (total > INT32_MAX) return set_error(GNNAGG_ERR_ARG, "gnnagg_dist_connect: more than 2^31 rows sent");
+    const int T = (int)total;
+    const cudaStream_t st = nullptr;
+    DT_TRY(cudaMalloc((void **)&d->ret_off, ((size_t)T + 1) * sizeof(int)));
+    DT_TRY(cudaMemsetAsync(d->ret_off, 0, sizeof(int), st));
+    d->ret_rows = 0;
+    if (T == 0) return GNNAGG_OK;
+    DT_TRY(cudaMalloc((void **)&d->ret_row, (size_t)T * sizeof(int)));
+    DT_TRY(cudaMalloc((void **)&d->ret_ent, (size_t)T * sizeof(unsigned long long)));
+    DT_TRY(cudaMalloc((void **)&s.keys, (size_t)T * sizeof(int)));
+    DT_TRY(cudaMalloc((void **)&s.keys_sorted, (size_t)T * sizeof(int)));
+    DT_TRY(cudaMalloc((void **)&s.counts, (size_t)T * sizeof(int)));
+    DT_TRY(cudaMalloc((void **)&s.num_runs, sizeof(int)));
+    DT_TRY(cudaMalloc((void **)&s.vals, (size_t)T * sizeof(unsigned long long)));
+    int at = 0;
+    for (int q = 0; q < d->world; ++q)
+        for (int c = 0; c < d->rounds; ++c) {
+            const int cnt = d->send_cnt[q][c];
+            if (cnt == 0) continue;
+            grad_return_fill_kernel<<<nblocks(cnt), 256, 0, st>>>(d->send_rows[q] + d->send_off[q][c], cnt, q,
+                                                                 d->peer_rows[q] + d->peer_slot[q][c], s.keys + at, s.vals + at);
+            at += cnt;
+            ++d->launches;
+        }
+    int bits = 1;
+    while (bits < 31 && (1ll << bits) < (int64_t)d->rows) ++bits;
+    size_t need = 0, b = 0;
+    DT_TRY(cub::DeviceRadixSort::SortPairs(nullptr, b, s.keys, s.keys_sorted, s.vals, d->ret_ent, T, 0, bits, st));
+    need = std::max(need, b);
+    DT_TRY(cub::DeviceRunLengthEncode::Encode(nullptr, b, s.keys_sorted, d->ret_row, s.counts, s.num_runs, T, st));
+    need = std::max(need, b);
+    DT_TRY(cub::DeviceScan::InclusiveSum(nullptr, b, s.counts, d->ret_off + 1, T, st));
+    need = std::max(need, b);
+    DT_TRY(cudaMalloc(&s.tmp, need ? need : 1));
+    b = need;
+    DT_TRY(cub::DeviceRadixSort::SortPairs(s.tmp, b, s.keys, s.keys_sorted, s.vals, d->ret_ent, T, 0, bits, st));  // stable
+    b = need;
+    DT_TRY(cudaMemsetAsync(s.counts, 0, (size_t)T * sizeof(int), st));
+    DT_TRY(cub::DeviceRunLengthEncode::Encode(s.tmp, b, s.keys_sorted, d->ret_row, s.counts, s.num_runs, T, st));
+    b = need;
+    DT_TRY(cub::DeviceScan::InclusiveSum(s.tmp, b, s.counts, d->ret_off + 1, T, st));
+    DT_TRY(cudaMemcpyAsync(&d->ret_rows, s.num_runs, sizeof(int), cudaMemcpyDeviceToHost, st));
+    DT_TRY(cudaGetLastError());
+    DT_TRY(cudaStreamSynchronize(st));
+    d->launches += 4;  // sort, encode, memset, scan
+    return GNNAGG_OK;
 }
 
 extern "C" {
@@ -608,6 +753,9 @@ int gnnagg_dist_create_rank(int rank, int world, const int64_t *shard_bounds, in
         if (cudaFuncSetAttribute(halo_push_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kPushBufs * kPushBatchBytes) != cudaSuccess)
             cudaGetLastError();
         if (const char *env = getenv("GNNAGG_PUSH_TMA")) d->push_tma = atoi(env) != 0;
+        if (cudaFuncGetAttributes(&attr, grad_wait_kernel) != cudaSuccess) cudaGetLastError();  // the backward step
+        if (cudaFuncGetAttributes(&attr, grad_signal_kernel) != cudaSuccess) cudaGetLastError();
+        if (cudaFuncGetAttributes(&attr, grad_return_kernel) != cudaSuccess) cudaGetLastError();
         dense_preload();
     }
     *out = d;
@@ -652,6 +800,8 @@ int gnnagg_dist_export(gnnagg_dist *d, void *blob)
     b.bytes = d->bytes;
     b.off_x[0] = d->off_x[0], b.off_x[1] = d->off_x[1], b.off_req = d->off_req, b.off_meta = d->off_meta;
     b.rounds = d->rounds;
+    b.backward = d->bwd_enabled ? 1 : 0;
+    b.off_g = d->off_g;
     // a handle is only needed by OTHER processes; a failure here (IPC not permitted) is reported at connect time
     if (cudaIpcGetMemHandle(&b.mem, d->base) != cudaSuccess) {
         cudaGetLastError();
@@ -705,6 +855,9 @@ int gnnagg_dist_connect(gnnagg_dist *d, const void *blobs)
         d->peer_rows[p] = (int)b.rows;
         // the rows p wants from this owner: per round c the slots [tab[c][rank], tab[c][rank + 1]) of ITS list; copied once
         if (b.rounds != d->rounds) return set_error(GNNAGG_ERR_ARG, "gnnagg_dist_connect: ranks disagree on the pipelining mode");
+        if (b.backward != (d->bwd_enabled ? 1 : 0))
+            return set_error(GNNAGG_ERR_ARG, "gnnagg_dist_connect: ranks disagree on gnnagg_dist_enable_backward");
+        d->peer_off_g[p] = b.off_g;
         int tab[kMaxRounds][kMaxWorld + 1];
         DT_TRY(cudaMemcpy(tab, d->peer_base[p] + b.off_meta, sizeof tab, cudaMemcpyDefault));
         int total_rows = 0;
@@ -725,6 +878,8 @@ int gnnagg_dist_connect(gnnagg_dist *d, const void *blobs)
         if (b.device == d->device) ++same;
     }
     d->same_device_ranks = same;
+    if (d->bwd_enabled)
+        if (int rc = build_return_tables(d)) return rc;
     d->connected = true;
     return GNNAGG_OK;
 }
@@ -833,13 +988,13 @@ int gnnagg_dist_set_graph(gnnagg_dist *d, const int *d_ptr, const int *d_idx, co
     for (int p = 0; p < W; ++p) b.stage_of[p] = d->stage_of[p];
 
     int *mark = nullptr, *pos = nullptr, *bad = nullptr, *idx_new = nullptr, *keys = nullptr, *item_row = nullptr, *first = nullptr,
-        *slot = nullptr;
+        *slot = nullptr, *t_perm = nullptr;
     void *tmp = nullptr;
     size_t tmp_bytes = 0;
     int rc = GNNAGG_OK;
     auto cleanup = [&]() {
         cudaFree(mark), cudaFree(pos), cudaFree(bad), cudaFree(idx_new), cudaFree(keys), cudaFree(item_row), cudaFree(first),
-            cudaFree(slot), cudaFree(tmp);
+            cudaFree(slot), cudaFree(tmp), cudaFree(t_perm);
     };
 #define SG_TRY(expr)                                                                             \
     do {                                                                                         \
@@ -927,6 +1082,10 @@ int gnnagg_dist_set_graph(gnnagg_dist *d, const int *d_ptr, const int *d_idx, co
         d->off_x[0] = d->off_req + req;
         d->off_x[1] = d->off_x[0] + xbuf;
         d->bytes = d->off_x[1] + xbuf;
+        if (d->bwd_enabled) {  // G of the backward: the size of one X buffer, so that slot s of G lines up with receive slot s
+            d->off_g = d->bytes;
+            d->bytes += xbuf;
+        }
         SG_TRY(cudaMalloc((void **)&d->base, d->bytes));
         SG_TRY(cudaMemsetAsync(d->base, 0, kFlagBytes + kMetaBytes, st));
         d->peer_base[d->rank] = d->base;
@@ -980,10 +1139,22 @@ int gnnagg_dist_set_graph(gnnagg_dist *d, const int *d_ptr, const int *d_idx, co
             dist_gather_val_kernel<<<nblocks(d->sl_cnt[s]), 256, 0, st>>>(d_val, d->sl_perm + d->sl_off[s], d->sl_val + d->sl_off[s],
                                                                         d->sl_cnt[s]);
     }
+    if (d->bwd_enabled) {
+        // the whole re-indexed block transposed (num_src = shard rows + receive slots), with its values in transposed order
+        rc = transpose_build_device(d_ptr, idx_new, item_row, items, n, m, n + (int)d->num_recv, &d->bw_ptr, &d->bw_idx, &t_perm, st);
+        if (rc != GNNAGG_OK) {
+            cleanup();
+            free_graph(d);
+            return rc;
+        }
+        SG_TRY(cudaMalloc((void **)&d->bw_val, me * sizeof(float)));
+        if (m > 0) dist_gather_val_kernel<<<nblocks(m), 256, 0, st>>>(d_val, t_perm, d->bw_val, m);
+        d->launches += 4 + (m > 0);  // iota, radix sort, rows, pointers; values
+    }
     SG_TRY(cudaGetLastError());
     SG_TRY(cudaStreamSynchronize(st));
     cleanup();
-    mark = pos = bad = idx_new = keys = item_row = first = slot = nullptr;
+    mark = pos = bad = idx_new = keys = item_row = first = slot = t_perm = nullptr;
     tmp = nullptr;
     cudaFree(d->sl_perm);  // only needed for the values
     d->sl_perm = nullptr;
@@ -993,6 +1164,16 @@ int gnnagg_dist_set_graph(gnnagg_dist *d, const int *d_ptr, const int *d_idx, co
         // stages run on their own CSR: the merged view of duplicate edges is not used across ranks (yet)
         if (rc == GNNAGG_OK) rc = gnnagg_set_merge_duplicates(d->stage[s], 1);
         if (rc == GNNAGG_OK) rc = gnnagg_set_val(d->stage[s], d->sl_val + d->sl_off[s]);
+        if (rc != GNNAGG_OK) {
+            free_graph(d);
+            return rc;
+        }
+    }
+    if (d->bwd_enabled) {
+        // an ordinary aggregator over the transposed block: gnnagg_gcn_run_rows runs its slot rows and its own rows apart
+        rc = gnnagg_create(d->bw_ptr, d->bw_idx, nullptr, nullptr, n + (int)d->num_recv, m, &d->bwd);
+        if (rc == GNNAGG_OK) rc = gnnagg_set_merge_duplicates(d->bwd, 1);  // as the stages: the CSR as built
+        if (rc == GNNAGG_OK) rc = gnnagg_set_val(d->bwd, d->bw_val);
         if (rc != GNNAGG_OK) {
             free_graph(d);
             return rc;
@@ -1013,6 +1194,8 @@ int gnnagg_dist_prepare(gnnagg_dist *d, int feat, void *stream)
     DeviceGuard guard(d->device);
     for (int s = 0; s < d->num_stages; ++s)
         if (int rc = gnnagg_prepare(d->stage[s], feat, stream)) return rc;
+    if (d->bwd)
+        if (int rc = gnnagg_prepare(d->bwd, feat, stream)) return rc;
     // A*X of the fused layer: allocated here rather than inside the first step for the same reason
     const size_t need = (size_t)d->rows * feat;
     if (need > d->ax_cap) {
@@ -1078,8 +1261,10 @@ int gnnagg_dist_check(gnnagg_dist *d)
     DT_TRY(cudaMemcpy(&err, &flags_of(d->base)->err, sizeof err, cudaMemcpyDeviceToHost));
     if (err) {
         char buf[160];
+        // forward: arrived (p), consumed (0x100 + q); backward: grad_ready (0x200 + q), grad_read (0x300 + p)
+        const uint32_t kind = err & 0x300u;
         snprintf(buf, sizeof buf, "halo protocol: rank %d gave up waiting for rank %u (%s flag, code 0x%x)", d->rank, err & 0xffu,
-                 (err & 0x100u) ? "consumed" : "arrived", err);
+                 kind == 0x300u ? "grad_read" : kind == 0x200u ? "grad_ready" : kind == 0x100u ? "consumed" : "arrived", err);
         return set_error(GNNAGG_ERR_STATE, buf);
     }
     return GNNAGG_OK;
@@ -1090,6 +1275,7 @@ int64_t gnnagg_dist_launch_count(const gnnagg_dist *d)
     if (!d) return 0;
     int64_t total = d->launches;
     for (int s = 0; s < d->num_stages; ++s) total += gnnagg_launch_count(d->stage[s]);
+    total += gnnagg_launch_count(d->bwd);
     return total;
 }
 
@@ -1354,6 +1540,83 @@ int gnnagg_dist_gcn_layer_host_bf16(gnnagg_dist *d, int buf, const uint16_t *h_X
                                     int feat_out, void *stream)
 {
     return dist_layer_host(d, buf, true, h_X, h_W, h_out, feat_in, feat_out, stream);
+}
+
+int gnnagg_dist_enable_backward(gnnagg_dist *d)
+{
+    if (!d) return set_error(GNNAGG_ERR_ARG, "gnnagg_dist_enable_backward: NULL handle");
+    if (d->base)
+        return set_error(GNNAGG_ERR_STATE, "gnnagg_dist_enable_backward: the rank already has a graph (enable comes before set_graph)");
+    d->bwd_enabled = true;
+    return GNNAGG_OK;
+}
+
+// One backward step on rank r (backward epoch e):
+//   1. wait until every owner has finished reading r's G of epoch e-1 (grad_read: write-after-read protection of G);
+//   2. G[rows, rows + num_recv) = slot rows of A^T dY: the partial sums of the remote sources, in receive-slot order;
+//   3. raise grad_ready[r] at every owner (also when nothing was written for it);
+//   4. dX = own rows of A^T dY, while the owners read G;
+//   5. wait for grad_ready of every peer;
+//   6. dX[u] += G_q[slot_q(u)] for the peers q that reference u, ascending q (grad_return_kernel, remote loads);
+//   7. raise grad_read[r] at every sender.
+// Launches of this function: 5 when world > 1, plus those of the two row-range runs of the transposed block.
+int gnnagg_dist_gcn_backward(gnnagg_dist *d, const float *dY, float *dX, int feat, void *stream)
+{
+    if (!d) return set_error(GNNAGG_ERR_ARG, "gnnagg_dist_gcn_backward: NULL handle");
+    if (!d->bwd_enabled)
+        return set_error(GNNAGG_ERR_STATE, "gnnagg_dist_gcn_backward: backward not enabled (gnnagg_dist_enable_backward before set_graph)");
+    if (!d->bwd) return set_error(GNNAGG_ERR_STATE, "gnnagg_dist_gcn_backward: no graph (gnnagg_dist_set_graph)");
+    if (!d->connected) return set_error(GNNAGG_ERR_STATE, "gnnagg_dist_gcn_backward: peers not connected (gnnagg_dist_connect)");
+    if (feat < 4 || (feat & 3) || feat > d->feat_cap)
+        return set_error(GNNAGG_ERR_ARG, "gnnagg_dist_gcn_backward: feat must be a multiple of 4, at most feat_cap");
+    if (d->rows > 0 && (!dY || !dX)) return set_error(GNNAGG_ERR_ARG, "gnnagg_dist_gcn_backward: NULL argument");
+    if (((uintptr_t)dY | (uintptr_t)dX) & 15) return set_error(GNNAGG_ERR_ARG, "gnnagg_dist_gcn_backward: dY and dX must be 16-byte aligned");
+    DeviceGuard guard(d->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    // as in the forward: a process that drives several ranks prepares every rank for a new width beforehand
+    if (d->prepared_feat != feat)
+        if (int rc = gnnagg_dist_prepare(d, feat, st)) return rc;
+    const int Wd = d->world, n = d->rows, S = (int)d->num_recv;
+    // dX = own rows of A^T dY (an edgeless block is written directly: its aggregator keeps no host row pointers)
+    auto own_rows = [&]() -> int {
+        if (n == 0) return GNNAGG_OK;
+        if (d->num_e == 0) {
+            DT_TRY(cudaMemsetAsync(dX, 0, (size_t)n * feat * sizeof(float), st));
+            return GNNAGG_OK;
+        }
+        return gnnagg_gcn_run_rows(d->bwd, dY, dX, feat, 0, 0, n, st);
+    };
+    if (Wd == 1) return own_rows();
+    HaloFlags *mine = flags_of(d->base);
+    PeerTable peers;
+    GradPeers gp;
+    memset(&peers, 0, sizeof peers);
+    memset(&gp, 0, sizeof gp);
+    for (int p = 0; p < Wd; ++p) {
+        peers.flags[p] = flags_of(d->peer_base[p]);
+        gp.g[p] = reinterpret_cast<const float4 *>(d->peer_base[p] + d->peer_off_g[p]);
+    }
+    const uint32_t others = (((Wd >= 32 ? 0u : (1u << Wd)) - 1u) & ~(1u << d->rank));
+    const uint32_t e = ++d->bepoch;
+    float *G = reinterpret_cast<float *>(d->base + d->off_g);
+    grad_wait_kernel<<<1, 32, 0, st>>>(mine->grad_read, others, e - 1u, &mine->err, 0x300u);
+    DT_TRY(cudaPeekAtLastError());
+    if (S > 0)
+        if (int rc = gnnagg_gcn_run_rows(d->bwd, dY, G, feat, 0, n, n + S, st)) return rc;
+    grad_signal_kernel<<<1, 32, 0, st>>>(peers, d->rank, Wd, 0, e);
+    DT_TRY(cudaPeekAtLastError());
+    if (int rc = own_rows()) return rc;
+    grad_wait_kernel<<<1, 32, 0, st>>>(mine->grad_ready, others, e, &mine->err, 0x200u);
+    DT_TRY(cudaPeekAtLastError());
+    const int F4 = feat / 4;
+    const int64_t threads = (int64_t)d->ret_rows * F4;
+    grad_return_kernel<<<(unsigned)std::max<int64_t>(1, (threads + 255) / 256), 256, 0, st>>>(
+        gp, d->ret_row, d->ret_off, d->ret_ent, reinterpret_cast<float4 *>(dX), d->ret_rows, F4);
+    DT_TRY(cudaPeekAtLastError());
+    grad_signal_kernel<<<1, 32, 0, st>>>(peers, d->rank, Wd, 1, e);
+    DT_TRY(cudaPeekAtLastError());
+    d->launches += 5;
+    return GNNAGG_OK;
 }
 
 }  // extern "C"

@@ -139,6 +139,8 @@ _SIGS = {
     "gnnagg_dist_profile_read": (C.c_int, [C.c_void_p, C.POINTER(C.c_float)]),
     "gnnagg_dist_check": (C.c_int, [C.c_void_p]),
     "gnnagg_dist_launch_count": (C.c_int64, [C.c_void_p]),
+    "gnnagg_dist_enable_backward": (C.c_int, [C.c_void_p]),
+    "gnnagg_dist_gcn_backward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
 }
 
 DIST_BLOB_BYTES = 256

@@ -334,9 +334,10 @@ class PeerHalo:
     driving several ranks, which connects them itself); otherwise the rank is created on the current device and
     connected to its peers through torch.distributed (any backend: the blobs are plain bytes).
     remote_stages = 0: one pass after all rows have arrived; R >= 1: stage 0 = local sources, then R groups of
-    owners accumulated as they land."""
+    owners accumulated as they land.  backward=True (on every rank alike) also readies gcn_backward: the transposed
+    block, a G buffer the size of one X buffer and the return tables."""
 
-    def __init__(self, ptr, idx, val, bounds, rank, world, feat_cap, remote_stages=1, group=None, handle=None):
+    def __init__(self, ptr, idx, val, bounds, rank, world, feat_cap, remote_stages=1, group=None, handle=None, backward=False):
         import ctypes as C
 
         import torch
@@ -357,6 +358,9 @@ class PeerHalo:
             self.h = h
         else:
             self.h = handle
+        self.backward = bool(backward)
+        if self.backward:
+            check(L.gnnagg_dist_enable_backward(self.h))
         check(L.gnnagg_dist_set_graph(self.h, _dp(ptr.contiguous()), _dp(idx.contiguous()), _dp(val.contiguous()), idx.numel(),
                                       int(remote_stages), _stream()))
         if handle is None and world > 1:
@@ -434,6 +438,14 @@ class PeerHalo:
                   _stream()))
         return H
 
+    def gcn_backward(self, dY, dX):
+        """dX = (A^T dY) on this rank's shard rows, dY and dX float32 [rows, feat].  Collective: every rank calls it
+        with the same width, as many times; needs backward=True at construction"""
+        from . import _f32, _stream, check, lib
+
+        check(lib().gnnagg_dist_gcn_backward(self.h, _f32(dY, "dY"), _f32(dX, "dX"), int(dY.shape[1]), _stream()))
+        return dX
+
     def gcn_layer_host(self, hX, hW, hH, buf=0):
         """pinned host X shard (float32 or bfloat16) and W -> host H (or A*X when hW is None), float32; copies inside,
         synchronises the stream"""
@@ -510,9 +522,9 @@ class LocalDist:
         self.handles = [C.c_void_p(self._hs[r]) for r in range(world)]
         self.ranks = [None] * world
 
-    def set_graph(self, rank, ptr, idx, val, remote_stages=1):
+    def set_graph(self, rank, ptr, idx, val, remote_stages=1, backward=False):
         self.ranks[rank] = PeerHalo(ptr, idx, val, self.bounds, rank, self.world, self.feat_cap, remote_stages,
-                                    handle=self.handles[rank])
+                                    handle=self.handles[rank], backward=backward)
         return self.ranks[rank]
 
     def connect(self):
@@ -533,6 +545,47 @@ class LocalDist:
         for h in self.handles:
             lib().gnnagg_dist_destroy(h)
         self.handles = []
+
+
+_dist_gcn_fn = None
+
+
+def _dist_gcn_function():
+    """the autograd Function behind dist_gcn_aggregate, defined on first use (this module imports torch lazily)"""
+    global _dist_gcn_fn
+    if _dist_gcn_fn is None:
+        import torch
+
+        class DistGCNAggregate(torch.autograd.Function):
+            @staticmethod
+            def forward(ctx, ph, X, buf):
+                F = X.shape[1]
+                ph.x(buf, F, X.dtype).copy_(X)
+                Y = torch.empty((ph.rows, F), device=X.device, dtype=torch.float32)
+                ph.gcn_run(Y, buf, F, dtype=X.dtype)
+                ctx.ph, ctx.x_dtype = ph, X.dtype
+                return Y
+
+            @staticmethod
+            def backward(ctx, dY):
+                dX = torch.empty(dY.shape, device=dY.device, dtype=torch.float32)
+                ctx.ph.gcn_backward(dY.contiguous(), dX)
+                return None, dX.to(ctx.x_dtype), None
+
+        _dist_gcn_fn = DistGCNAggregate
+    return _dist_gcn_fn
+
+
+def dist_gcn_aggregate(ph, X, buf=0):
+    """Y = A_block X across ranks as a differentiable op: X is this rank's shard [rows, F] (float32 or bfloat16), copied
+    into shard buffer `buf` of the PeerHalo `ph` (made with backward=True); Y is float32.  The backward is
+    gnnagg_dist_gcn_backward, dX computed in float32 and rounded once to X's dtype (a bf16 shard needs nothing else: the
+    backward never reads X).  A layer is this op followed by torch.matmul with W.
+
+    The op is collective in both directions: every rank runs its forward, and later its backward, the same number of
+    times with the same width.  In one process driving several ranks (LocalDist), each rank's forward must run on its
+    own stream, as gcn_run already requires; autograd runs each backward on the stream of its forward."""
+    return _dist_gcn_function().apply(ph, X, buf)
 
 
 def stage_ends(world, R):

@@ -411,6 +411,30 @@ int gnnagg_dist_profile_read(gnnagg_dist *d, float *ms /* [4] */);
 /* GNNAGG_ERR_STATE if a kernel of this rank gave up waiting for a peer (bounded spin, 20 s); synchronous */
 int gnnagg_dist_check(gnnagg_dist *d);
 int64_t gnnagg_dist_launch_count(const gnnagg_dist *d);
+/* ---- backward across ranks: dX = A^T dY ------------------------------------------------------------------
+ * gnnagg_dist_enable_backward  before gnnagg_dist_set_graph, on every rank of the group alike (GNNAGG_ERR_STATE after
+ *                              set_graph; connect rejects a group whose ranks disagree, GNNAGG_ERR_ARG).  set_graph then
+ *                              also keeps the re-indexed block transposed on the GPU (rows = shard rows + receive slots)
+ *                              and a G buffer the size of one X buffer inside the peer-visible allocation; connect builds
+ *                              the return tables.  Off by default: a forward-only group allocates what it did before.
+ * gnnagg_dist_gcn_backward     dX = (A^T dY) restricted to this rank's shard rows, for the aggregation of
+ *                              gnnagg_dist_gcn_run / _gcn_layer (edge values of set_graph).  dY, dX: [rows, feat] fp32,
+ *                              16-byte aligned, distinct; feat a multiple of 4 <= feat_cap; dX is overwritten.  Collective:
+ *                              every rank calls it with the same feat, the same number of times.  Asynchronous on `stream`.
+ *                              Each rank writes the partial sums of the remote sources it references into its own G
+ *                              (receive-slot order); each owner reads the rows meant for it with remote loads and adds
+ *                              them to its own contribution in ascending peer order: no atomics, bit-reproducible for a
+ *                              given (world, remote_stages), independent of arrival timing; not bit-equal to
+ *                              gnnagg_gcn_backward (different grouping of the sums).  Its flags and epochs are separate
+ *                              from the forward's, so forward and backward steps may interleave.  A width other than the
+ *                              last prepared one needs gnnagg_dist_prepare on every rank first when one process drives
+ *                              several ranks (as for the forward).  Launches: 5 per step when world > 1, plus those of the
+ *                              row-range runs of the transposed block (folded into gnnagg_dist_launch_count).
+ *                              Errors, reported before any launch: GNNAGG_ERR_STATE when backward is not enabled, there
+ *                              is no graph or the rank is not connected; GNNAGG_ERR_ARG for a bad feat, a NULL pointer with
+ *                              rows > 0 or a misaligned pointer. */
+int gnnagg_dist_enable_backward(gnnagg_dist *d);
+int gnnagg_dist_gcn_backward(gnnagg_dist *d, const float *dY, float *dX, int feat, void *stream);
 
 /* ------------------------------------------------------------------------------------------
  * Host-buffer entry points (what a caller holding HOST arrays uses; bench.py's e2e number).
